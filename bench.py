@@ -13,14 +13,24 @@ headline, every N also times the ROW-SHARDED table + tied head of configs[3] and
 ``--impl reference`` times the reference's own CPU implementation of the path (the
 oracle graph: stock torch ops + the Hugging Face encoder, all host threads) on a
 bounded sample of the same workload.
+
+``--dump-outputs DIR`` writes what the timed path returned in its last timed step as
+``DIR/<name>.npy`` (see ``dump_outputs``).  Inputs, weights and random draws are seeded, so
+two builds run with the same arguments can be compared output for output.
+
+The benchmark writes nothing into the source tree (which may be read-only): no bytecode
+caches, and its one scratch file goes to the system's temporary directory.
 """
 import argparse
 import json
 import os
 import subprocess
 import sys
+import tempfile
 import threading
 import time
+
+sys.dont_write_bytecode = True
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 for _p in (ROOT, os.path.join(ROOT, "oracle"), os.path.join(ROOT, "tests")):
@@ -380,7 +390,11 @@ def main():
                          "optimizer step); not BASELINE.json's metric -- the line says so in `metric`")
     ap.add_argument("--optimizer", choices=["sgd", "adamw"], default="sgd",
                     help="with --train: torch.optim.SGD, or FusedAdamW (the t4r_train_adamw kernel)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the outputs of the last timed step as DIR/<name>.npy (float32 / float64, under 64 MB)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     cfg = dict(CONFIGS[args.workload])
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
@@ -403,7 +417,7 @@ def main():
     if args.impl == "reference":
         if rank != 0:
             return
-        steps = max(1, min(args.steps, 5))
+        steps = args.steps
         warm = 1
         v, med, threads, b_run = time_oracle_cpu(cfg, args.cpu_sessions, steps, warm)
         line = {"impl": "reference", "metric": METRIC, "value": v, "unit": "sessions/s", "n_gpus": args.gpus,
@@ -529,6 +543,54 @@ def _gather_time(model, cfg, batches, K):
     return ms, nbytes
 
 
+DUMP_PREDICTION_BYTES = 48 << 20   # the sampled prediction rows; with loss and labels the dump stays under 64 MB
+
+
+def dump_outputs(path, loss, task, train_step=None, seed=0):
+    """Write what a caller of the timed step received from its last call as ``path/<name>.npy``: ``loss``, ``labels``
+    (the targets of the masked positions, in row order) and, where the path materialises them, ``predictions`` -- the
+    rows of the [T, V] scores (or [T, 1 + S] with sampled softmax) at a fixed seeded sample of label rows, whose
+    indices are ``prediction_rows``; the whole matrix does not fit.  Floats are stored as float32, integers as
+    float64, which holds them exactly."""
+    import numpy as np
+
+    if train_step is not None:
+        arrays = {"loss": loss, "labels": train_step.labels[:train_step.T]}
+    else:
+        arrays = {"loss": loss, "labels": task._lazy_labels()}
+        if "xt_planes" in task._last:   # over a row-sharded table the path does not materialise predictions
+            arrays.update(_prediction_rows(task, seed))
+    os.makedirs(path, exist_ok=True)
+    for name, t in arrays.items():
+        t = t.detach().cpu()
+        np.save(os.path.join(path, f"{name}.npy"), t.numpy().astype(np.float32 if t.is_floating_point() else np.float64))
+
+
+def _prediction_rows(task, seed):
+    """``predictions`` of the task's last forward at a seeded sample of its label rows: the task's own materialisation
+    pointed at a copy of those rows (zero-padded to whole 128-row tiles), so the scores are computed as for all rows."""
+    st = task._last
+    T = int(st["count"].item())
+    cols = 1 + st["neg"].numel() if st["sampled"] else task.output_weight().shape[0]
+    R = min(T, max(1, DUMP_PREDICTION_BYTES // (4 * cols)))
+    rows = torch.randperm(T, generator=torch.Generator().manual_seed(seed))[:R].sort().values
+    idx = rows.to(st["labels"].device)
+    planes = st["xt_planes"]
+    sub_planes = torch.zeros((planes.shape[0], (R + 127) // 128 * 128, planes.shape[2]), dtype=planes.dtype,
+                             device=planes.device)
+    sub_planes[:, :R] = planes[:, idx]
+    sub = dict(st, xt_planes=sub_planes, labels=st["labels"][idx],
+               count=torch.full((1,), R, dtype=torch.int32, device=idx.device))
+    if st["sampled"]:
+        sub["pos"] = st["pos"][idx]
+    task._last = sub
+    try:
+        predictions = task._lazy_predictions()
+    finally:
+        task._last = st
+    return {"predictions": predictions, "prediction_rows": rows}
+
+
 def run_workload(args, cfg, dev, rank, world, local_rank, config_desc, peaks, peak_kind, headline):
     import transformers4rec_b200 as t4r
     from transformers4rec_b200 import ops
@@ -590,7 +652,7 @@ def run_workload(args, cfg, dev, rank, world, local_rank, config_desc, peaks, pe
     e0.record()
     for i in range(K):
         ops.HEAD_EVENTS = evs[i]
-        step(devs[i % N_ROTATE])
+        loss_last = step(devs[i % N_ROTATE])
     e1.record()
     barrier()
     ops.HEAD_EVENTS = None
@@ -600,6 +662,8 @@ def run_workload(args, cfg, dev, rank, world, local_rank, config_desc, peaks, pe
     head_ms = sorted(a.elapsed_time(b) for a, b in evs)
     head_ms_avg = sum(head_ms) / len(head_ms)
     T = train_step.T if train_step is not None else int(task._last["count"].item())
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, loss_last, task, train_step)  # before any later forward replaces task._last
 
     # --- optional: the same step captured once and replayed from a CUDA graph (no host work at all)
     graph_ms = None
@@ -796,7 +860,7 @@ def run_sharded_leg(args, name, dev, rank, world, peaks):
     def step(i):
         with torch.no_grad():
             return model(devs[i % N_ROTATE], training=True)["loss"]
-    K = max(3, min(args.steps, 10))
+    K = args.steps
     for i in range(3):
         step(i)
     dist.barrier(); torch.cuda.synchronize()
@@ -868,7 +932,7 @@ def run_sharded_leg(args, name, dev, rank, world, peaks):
                 "head_frac_of_bf16_peak": head_flops / (head_ms * 1e-3) / 1e12 / peak_tf,
                 "nccl_collectives_per_step": colls, "scaling": "weak"})
     # own efficiency v_N / (N * v_1): v_1 is read from the N = 1 run of the same session when it left its note
-    note = os.path.join(ROOT, ".bench_sharded_n1.json")
+    note = os.path.join(tempfile.gettempdir(), "t4r_bench_sharded_n1.json")
     try:
         if rank == 0 and world == 1:
             prev = {}

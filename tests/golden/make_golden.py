@@ -1,8 +1,9 @@
 #!/usr/bin/env python
 """Generate golden input/output vectors by executing the UPSTREAM reference code.
 
-Runs only in the authoring container (needs /root/reference; the GPU box does not
-have it).  The reference package cannot be imported as a whole here (merlin-*,
+Needs a source checkout of NVIDIA-Merlin/Transformers4Rec, named by the environment
+variable T4R_UPSTREAM_SRC; the tests only read the stored vectors.  The reference
+package cannot be imported as a whole (merlin-*,
 betterproto, torchmetrics are absent and HF 5.5 dropped symbols it imports;
 SURVEY.md §8c), so this script loads the individual upstream source files for the
 arithmetic of the hot path -- masking.py, ranking_metric.py, the sampler / head in
@@ -16,7 +17,9 @@ position, k = floor(u*n)), so the very same draws can be fed to the oracle and t
 CUDA kernels.  Nothing from the reference is copied into this repository: only
 tensors it produced.
 
-Usage:  python tests/golden/make_golden.py     (writes tests/golden/*.pt)
+Usage:  T4R_UPSTREAM_SRC=<checkout> python tests/golden/make_golden.py     (writes tests/golden/*.pt)
+
+Every stored file stays under 1 MB; the head's vocabulary (Vh) and label rows (Th) are sized for that.
 """
 import importlib
 import os
@@ -26,7 +29,7 @@ import types
 import numpy as np
 import torch
 
-REF = "/root/reference"
+REF = os.environ.get("T4R_UPSTREAM_SRC", "")
 HERE = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, os.path.join(os.path.dirname(os.path.dirname(HERE)), "oracle"))
 import t4r_oracle as O  # noqa: E402  (only for the uniform->draw helpers, so both sides share them)
@@ -168,7 +171,7 @@ class patched_draws:
 
 
 def main():
-    assert os.path.isdir(REF), "the upstream reference is only mounted in the authoring container"
+    assert os.path.isdir(REF), "set T4R_UPSTREAM_SRC to a source checkout of NVIDIA-Merlin/Transformers4Rec"
     install_stubs()
     # utils/torch_utils.py imports the four masking classes at class-body time (a cycle the
     # real package resolves through its __init__ order): satisfy it with placeholders first
@@ -220,7 +223,7 @@ def main():
                      "known_answer_recall": torch.tensor([0.3333, 0.3333, 0.6667, 0.6667])}
 
     # ---------------------------------------------------------------- sampler + head
-    Vh, De, Th, S = 3001, 32, 50, 200
+    Vh, De, Th, S = 1001, 32, 32, 200
     sampler = ptask.LogUniformSampler(max_n_samples=S, max_id=Vh, min_id=1, unique_sampling=True)
     xt = torch.randn((Th, De), generator=g)
     W = torch.randn((Vh, De), generator=g) * 0.1

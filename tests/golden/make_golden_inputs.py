@@ -55,7 +55,7 @@ class patched_ssn_draws:
 
 
 def main():
-    assert os.path.isdir(G.REF), "the upstream reference is only mounted in the authoring container"
+    assert os.path.isdir(G.REF), "set T4R_UPSTREAM_SRC to a source checkout of NVIDIA-Merlin/Transformers4Rec"
     agg, emb, trf, rank = load_upstream()
     g = torch.Generator().manual_seed(4321)
     out = {}

@@ -504,25 +504,33 @@ def test_attention_backward_host_twin_matches_autograd(L, H, dh):
 def test_descriptor_encodings_match_the_vendored_cutlass_headers(tmp_path):
     """tests/native/desc_check.cu: this repo's instruction descriptors (bf16 -- proven on hardware --, fp16 and e4m3 of
     the 2-unit product) against cute::UMMA::make_instr_desc, and the K-major SW128 / SW64 shared-memory descriptors
-    against cute::UMMA::SmemDescriptor's bit fields.  Skipped where nvcc or the headers are absent."""
+    against cute::UMMA::SmemDescriptor's bit fields: always against CuTe's values stored in
+    tests/golden/umma_descriptors.json, and against the headers themselves where an installed package vendors them."""
     import glob
+    import json
     import os
+    import re
     import shutil
     import subprocess
     import sys
     nvcc = shutil.which("nvcc") or "/usr/local/cuda/bin/nvcc"
     incs = glob.glob(os.path.join(sys.prefix, "lib", "python*", "site-packages", "flashinfer", "data", "cutlass", "include"))
-    if not os.path.exists(nvcc) or not incs:
-        pytest.skip("nvcc or the vendored CUTLASS headers are not available")
     root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-    exe = str(tmp_path / "desc_check")
-    cmd = [nvcc, "-std=c++17", "-w", "-gencode", "arch=compute_100a,code=sm_100a", "-I" + incs[0],
-           "-I" + os.path.join(root, "transformers4rec_b200", "csrc"), "-o", exe, os.path.join(root, "tests", "native", "desc_check.cu")]
-    res = subprocess.run(cmd, capture_output=True, text=True, timeout=600)
-    assert res.returncode == 0, res.stderr[-2000:]
-    run = subprocess.run([exe], capture_output=True, text=True, timeout=60)
-    assert run.returncode == 0 and "MISMATCH" not in run.stdout, run.stdout
-    assert run.stdout.count(" ok") >= 17
+    with open(os.path.join(root, "tests", "golden", "umma_descriptors.json")) as f:
+        want = json.load(f)["cute"]
+    for inc in [None] + incs[:1]:
+        exe = str(tmp_path / ("desc_check_cute" if inc else "desc_check"))
+        cmd = [nvcc, "-std=c++17", "-w", "-gencode", "arch=compute_100a,code=sm_100a"] + (["-I" + inc] if inc else []) + [
+               "-I" + os.path.join(root, "transformers4rec_b200", "csrc"), "-o", exe,
+               os.path.join(root, "tests", "native", "desc_check.cu")]
+        res = subprocess.run(cmd, capture_output=True, text=True, timeout=600)
+        assert res.returncode == 0, res.stderr[-2000:]
+        run = subprocess.run([exe], capture_output=True, text=True, timeout=60)
+        assert run.returncode == 0 and "MISMATCH" not in run.stdout, run.stdout
+        ours = dict(re.findall(r"^(.*?)\s+ours ([0-9a-f]+)", run.stdout, flags=re.M))
+        assert ours == want, run.stdout
+        if inc:
+            assert run.stdout.count(" ok") == len(want)
 
 
 def test_every_c_abi_call_site_matches_its_ctypes_signature():

@@ -170,6 +170,40 @@ def test_bench_workload_builders_train_like_the_oracle(monkeypatch, cfg):
     assert (task.task_block is not None) == (cfg["De"] != cfg["d"])
 
 
+@pytest.mark.parametrize("sampled", [0, 300], ids=["full-softmax", "sampled-softmax"])
+def test_bench_dump_outputs_are_what_the_caller_received(monkeypatch, tmp_path, sampled):
+    """bench.py --dump-outputs: loss, labels and a seeded sample of prediction rows as .npy files (floats float32,
+    integers float64), equal to what the forward returned; the same seed picks the same rows."""
+    import importlib.util
+    import os
+    import numpy as np
+    D.install(monkeypatch)
+    root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+    spec = importlib.util.spec_from_file_location("bench_mod6", os.path.join(root, "bench.py"))
+    bench = importlib.util.module_from_spec(spec)
+    spec.loader.exec_module(bench)
+    cfg = dict(V=2001, De=32, d=32, H=2, NL=1, L=12, B=8, arch="xlnet", masking="mlm", sampled=sampled, label="test")
+    model = bench.build_product_model(cfg, torch.device("cpu"))
+    task = model.heads[0].prediction_task_dict["next-item"]
+    with torch.no_grad():
+        out = model(bench.synth_batch(cfg["B"], cfg["L"], cfg, seed=0), training=True)
+        preds, labels = out["predictions"], out["labels"]
+        T = labels.numel()
+        monkeypatch.setattr(bench, "DUMP_PREDICTION_BYTES", 4 * 5 * preds.shape[1])   # room for 5 of the T rows
+        for d in ("a", "b"):
+            bench.dump_outputs(str(tmp_path / d), out["loss"], task)
+    got = {n: np.load(tmp_path / "a" / f"{n}.npy") for n in ("loss", "labels", "predictions", "prediction_rows")}
+    assert sorted(os.listdir(tmp_path / "a")) == sorted(f"{n}.npy" for n in got)
+    assert [got[n].dtype for n in got] == [np.float32, np.float64, np.float32, np.float64]
+    assert float(got["loss"]) == out["loss"].item() and np.array_equal(got["labels"], labels.numpy())
+    rows = torch.from_numpy(got["prediction_rows"]).long()
+    assert T > 5 and rows.numel() == 5 and bool((rows.diff() > 0).all()) and int(rows.max()) < T
+    assert np.allclose(got["predictions"], preds[rows].numpy(), atol=1e-5)
+    for n in got:
+        assert np.array_equal(np.load(tmp_path / "b" / f"{n}.npy"), got[n])
+    assert int(task._last["count"].item()) == T          # the task's state is left as the forward left it
+
+
 def test_permutation_language_modeling_flow(monkeypatch):
     """masking="plm" end to end (kernels = doubles): labels / masks / side channels, training and evaluation loss
     against the oracle graph, whose encoder is HF XLNet's two-stream forward with perm_mask + target_mapping."""
