@@ -377,7 +377,7 @@ def plm_apply_mask_to_inputs(x, mask_schema, masked_item_embedding, training=Fal
 def hf_encoder_forward_plm(model, x: torch.Tensor, perm_mask: torch.Tensor, target_mapping: torch.Tensor) -> torch.Tensor:
     """block/transformer.py:179-199 with masking.transformer_arguments = {target_mapping, perm_mask} (masking.py:739-740):
     HF returns the query stream g (one row per target position) as output[0]."""
-    return model(inputs_embeds=x, perm_mask=perm_mask.float(), target_mapping=target_mapping.float())[0]
+    return model(inputs_embeds=x, perm_mask=perm_mask.to(x.dtype), target_mapping=target_mapping.to(x.dtype))[0]
 
 
 # --------------------------------------------------------------------------- #
@@ -468,7 +468,7 @@ def xlnet_forward_restated(x: torch.Tensor, sd: Dict[str, torch.Tensor], n_layer
     B, L, d = x.shape
     H = n_head
     dh = d // H
-    pos = xlnet_relative_positions(L, d)  # [2L, d]
+    pos = xlnet_relative_positions(L, d).to(x.dtype)  # [2L, d]
     scale = 1.0 / math.sqrt(dh)
     D = drop if drop is not None else (lambda site, t: t)
     h = D(0, x)
@@ -775,7 +775,7 @@ class OracleSessionModel(torch.nn.Module):
             h = hf_encoder_forward(self.transformer, x)
         hs = h
         if self.task_block is not None:
-            h = self.task_block(h.float())
+            h = self.task_block(h.to(self.task_block.weight.dtype))
         x_t, y = select_targets(h, labels)
         W = self.item_table()
         if self.sampled_softmax and training:
