@@ -4,8 +4,8 @@
 // flashinfer/data/cutlass/include) it also prints CuTe's and compares.  The test holds our encodings to CuTe's values
 // as stored in tests/golden/umma_descriptors.json, so the check does not need the headers.
 //   instruction descriptor: cute::UMMA::make_instr_desc<A, B, float, M, N, K-major, K-major>()
-//   shared-memory descriptor: the bit fields of cute::UMMA::SmemDescriptor filled with the K-major SWIZZLE_128B /
-//   SWIZZLE_64B canonical values (start address >> 4, LBO = 1 unit, SBO = 8 rows * row bytes, version 1)
+//   shared-memory descriptor: the bit fields of cute::UMMA::SmemDescriptor filled with the K-major SWIZZLE_128B
+//   canonical values (start address >> 4, LBO = 1 unit, SBO = 8 rows * row bytes, version 1)
 #include <cstdio>
 #include "t4r_common.cuh"
 
@@ -36,7 +36,7 @@ static uint64_t cute_sw(uint32_t addr, int sbo_bytes, UMMA::LayoutType lt) {
 #define CUTE(expr) 0
 #endif
 
-// the device helpers restated for the host (same arithmetic as umma_desc_sw128 / umma_desc_sw64)
+// the device helper restated for the host (same arithmetic as umma_desc_sw128)
 static uint64_t ours_sw(uint32_t addr, int sbo_bytes, int layout) {
   uint64_t d = 0;
   d |= static_cast<uint64_t>((addr >> 4) & 0x3FFFu);
@@ -69,8 +69,6 @@ int main() {
   for (uint32_t addr : {0x0u, 0x400u, 0x8460u, 0x3fc20u}) {
     snprintf(what, sizeof what, "smem desc K-major SW128 @%05x", addr);
     CHECK64(ours_sw(addr, 1024, 2), cute_sw(addr, 1024, UMMA::LayoutType::SWIZZLE_128B), what);
-    snprintf(what, sizeof what, "smem desc K-major SW64 @%05x", addr);
-    CHECK64(ours_sw(addr, 512, 4), cute_sw(addr, 512, UMMA::LayoutType::SWIZZLE_64B), what);
   }
   return bad;
 }

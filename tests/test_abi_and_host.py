@@ -503,7 +503,7 @@ def test_attention_backward_host_twin_matches_autograd(L, H, dh):
 
 def test_descriptor_encodings_match_the_vendored_cutlass_headers(tmp_path):
     """tests/native/desc_check.cu: this repo's instruction descriptors (bf16 -- proven on hardware --, fp16 and e4m3 of
-    the 2-unit product) against cute::UMMA::make_instr_desc, and the K-major SW128 / SW64 shared-memory descriptors
+    the 2-unit product) against cute::UMMA::make_instr_desc, and the K-major SW128 shared-memory descriptor
     against cute::UMMA::SmemDescriptor's bit fields: always against CuTe's values stored in
     tests/golden/umma_descriptors.json, and against the headers themselves where an installed package vendors them."""
     import glob

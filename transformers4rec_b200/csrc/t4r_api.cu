@@ -8,13 +8,8 @@
 
 #include "t4r_common.cuh"
 #include <stddef.h>
-#include <mutex>
 
 #include "t4r_internal.h"
-
-#ifndef T4R_FFN_FUSED_DEFAULT
-#define T4R_FFN_FUSED_DEFAULT 1
-#endif
 
 namespace t4r {
 
@@ -158,14 +153,6 @@ extern "C" int t4r_ffn_fwd(const void* x_planes, int64_t M, int d, int hidden, c
 // ----------------------------------------------------------------------------
 // XLNet encoder
 // ----------------------------------------------------------------------------
-// T4R_FFN_FUSED=0 selects the two-GEMM feed-forward (intermediate planes through HBM) instead of the
-// fused kernel that keeps the GELU'd intermediate in TMEM.
-static bool use_ffn_fused(int d) {
-  int on = T4R_FFN_FUSED_DEFAULT;  // read per call (tests toggle it)
-  if (const char* e = getenv("T4R_FFN_FUSED")) on = atoi(e);
-  return on && ffn_fused_supported(d, 4 * d);
-}
-
 extern "C" size_t t4r_xlnet_encoder_workspace_bytes(int B, int L, int d, int n_head) {
   (void)n_head;
   const size_t M = static_cast<size_t>(B) * L;
@@ -176,42 +163,9 @@ extern "C" size_t t4r_xlnet_encoder_workspace_bytes(int B, int L, int d, int n_h
   b += pad256(2 * M * d * 2);        // attention output planes
   b += pad256(M * d * 4);            // h1 fp32
   b += pad256(2 * M * d * 2);        // h1 planes
-  b += pad256(2 * M * 4 * d * 2);    // ff planes
   b += pad256(2 * M * d * 2);        // x planes (when split internally)
   b += 2 * (pad256(M * d * 4) + pad256(2 * M * d * 2));  // layer io ping-pong
   return b + 1024;
-}
-
-// side streams + fork / join events of the row-part scheme below, one set per device, created on first use
-#ifndef T4R_ENC_PARTS_DEFAULT
-#define T4R_ENC_PARTS_DEFAULT 1
-#endif
-constexpr int kMaxEncParts = 4;
-struct EncStreams {
-  cudaStream_t side[kMaxEncParts - 1];
-  cudaEvent_t fork, join[kMaxEncParts - 1];
-};
-static EncStreams* enc_streams() {
-  static std::mutex mu;
-  static EncStreams* per_dev[64] = {nullptr};
-  int dev = 0;
-  if (cudaGetDevice(&dev) != cudaSuccess || dev < 0 || dev >= 64) return nullptr;
-  std::lock_guard<std::mutex> lk(mu);
-  if (!per_dev[dev]) {
-    EncStreams* es = new EncStreams();
-    bool ok = cudaEventCreateWithFlags(&es->fork, cudaEventDisableTiming) == cudaSuccess;
-    for (int i = 0; i < kMaxEncParts - 1 && ok; ++i)
-      ok = cudaStreamCreateWithFlags(&es->side[i], cudaStreamNonBlocking) == cudaSuccess &&
-           cudaEventCreateWithFlags(&es->join[i], cudaEventDisableTiming) == cudaSuccess;
-    if (!ok) { delete es; return nullptr; }
-    per_dev[dev] = es;
-  }
-  return per_dev[dev];
-}
-static int enc_parts_default() {
-  int n = T4R_ENC_PARTS_DEFAULT;
-  if (const char* e = getenv("T4R_ENC_PARTS")) n = atoi(e);   // read per call (tests and A/B runs toggle it)
-  return n < 1 ? 1 : (n > kMaxEncParts ? kMaxEncParts : n);
 }
 
 // plm_mask != nullptr: the two-stream PLM forward -- B counts the stacked row sessions (2 x the real batch: h rows, then
@@ -256,7 +210,6 @@ static int xlnet_encoder_impl(const t4r_xlnet_layer* layers, int n_layer, int B,
   const bool tc_attn = !force_simt && attn_mma_supported(L, d, n_head, true);
   __nv_bfloat16* qkv_p = reinterpret_cast<__nv_bfloat16*>(qkv);  // same bytes: [2, M, 3d] bf16
   __nv_bfloat16* h1_p = ar.take<__nv_bfloat16>(2 * M * d);
-  __nv_bfloat16* ff_p = ar.take<__nv_bfloat16>(2 * M * 4 * d);
   __nv_bfloat16* x_p_own = ar.take<__nv_bfloat16>(2 * M * d);
   float* io_f[2];
   __nv_bfloat16* io_p[2];
@@ -280,30 +233,6 @@ static int xlnet_encoder_impl(const t4r_xlnet_layer* layers, int n_layer, int B,
     for (int li = 0; li < n_layer; ++li) wrs[li] = layers[li].wr;
     T4R_TRY(launch_rel_pos_proj(wrs, n_layer, L, d, rbuf, tc_attn ? r_p : nullptr, s));
   }
-  // Row parts on concurrent streams.  Every kernel of a layer works on whole sessions and on nothing but its own rows,
-  // so the batch can be cut into `nparts` session ranges whose layer chains are independent: they are enqueued on
-  // separate streams, and while one part's persistent GEMM drains its last (partial) wave of 128-row tiles the SMs it
-  // has left are picked up by the other part's next kernel.  With one part the FFN runs 320 tiles on 148 SMs (2.16
-  // waves: 28 % of the kernel is the tail of the third wave); two parts fill those tails with each other's work.
-  // T4R_ENC_PARTS (default T4R_ENC_PARTS_DEFAULT); the two-stream PLM form stays in one part.
-  int nparts = 1;
-  if (!plm_mask) {
-    nparts = enc_parts_default();
-    while (nparts > 1 && (B % nparts != 0 || (static_cast<int64_t>(B) / nparts) * L < 4 * 128)) --nparts;
-  }
-  cudaStream_t ps[kMaxEncParts];
-  ps[0] = s;
-  if (nparts > 1) {
-    EncStreams* es = enc_streams();
-    T4R_REQUIRE(es != nullptr, "xlnet_encoder: could not create the side streams");
-    T4R_CUDA(cudaEventRecord(es->fork, s));
-    for (int p = 1; p < nparts; ++p) {
-      ps[p] = es->side[p - 1];
-      T4R_CUDA(cudaStreamWaitEvent(ps[p], es->fork, 0));
-    }
-  }
-  const int Bp = B / nparts;
-  const int64_t Mp = static_cast<int64_t>(Bp) * L;
   const float* in_f = x_f32;
   const __nv_bfloat16* in_p = cur_p;
   for (int li = 0; li < n_layer; ++li) {
@@ -313,85 +242,56 @@ static int xlnet_encoder_impl(const t4r_xlnet_layer* layers, int n_layer, int B,
     const __nv_bfloat16* r_p_l = r_p + static_cast<size_t>(li) * 4 * L * d;
     float* dst_f = last ? out_f32 : nullptr;
     __nv_bfloat16* dst_p = last ? static_cast<__nv_bfloat16*>(out_planes) : io_p[li & 1];
-    for (int part = 0; part < nparts; ++part) {
-      cudaStream_t sp = ps[part];
-      const int64_t r0 = part * Mp;   // first row of the part
-      // Q | K | V projections (HF:xlnet:253-259), one GEMM over the fused [3d, d] weight
-      {
-        GemmProblem pb;
-        pb.M = Mp; pb.N = 3 * d; pb.Kp = d;
-        pb.a_planes = in_p + r0 * d; pb.a_rows = M;
-        pb.b_planes = static_cast<const __nv_bfloat16*>(w.wqkv_planes); pb.b_rows = 3 * d;
-        GemmEpilogue ep;
-        if (tc_attn) { ep.out_planes = qkv_p + r0 * 3 * d; ep.ldpl = 3 * d; ep.plane_stride = M * 3 * d; }
-        else { ep.out_f32 = qkv + r0 * 3 * d; ep.ldo = 3 * d; }
-        T4R_TRY(launch_gemm(pb, ep, sp));
-      }
-      // relative attention core (HF:xlnet:95-140)
-      if (plm_mask) {
-        T4R_REQUIRE(tc_attn, "xlnet_encoder_plm: the FFMA attention fallback has no two-stream form (unset T4R_ATTN_SIMT)");
-        T4R_TRY(launch_attn_mma_plm(qkv_p, M * 3 * d, r_p_l, static_cast<int64_t>(2) * L * d, w.r_w_bias, w.r_r_bias, B / 2,
-                                    L, d, n_head, attn_p, M * d, plm_mask, sp));
-      } else if (tc_attn)
-        T4R_TRY(launch_attn_mma(true, qkv_p + r0 * 3 * d, M * 3 * d, r_p_l, static_cast<int64_t>(2) * L * d, w.r_w_bias,
-                                w.r_r_bias, Bp, L, d, n_head, attn_p + r0 * d, M * d, sp));
-      else
-        T4R_TRY(launch_xlnet_attn(qkv + r0 * 3 * d, rbuf_l, w.r_w_bias, w.r_r_bias, Bp, L, d, n_head, attn_p + r0 * d, M * d, sp));
-      // post_attention: h1 = LN(x + attn @ Wo^T) (HF:xlnet:142-152)
-      {
-        GemmProblem pb;
-        pb.M = Mp; pb.N = d; pb.Kp = d;
-        pb.a_planes = attn_p + r0 * d; pb.a_rows = M;
-        pb.b_planes = static_cast<const __nv_bfloat16*>(w.wo_planes); pb.b_rows = d;
-        GemmEpilogue ep;
-        // residual: the caller's fp32 x for the first layer, afterwards the split planes of the
-        // previous layer's output (hi + lo, exact to 16 mantissa bits) -- no fp32 copy of the
-        // residual stream is written between layers (the store path bounds these epilogues)
-        if (in_f) { ep.residual = in_f + r0 * d; ep.ldr = d; }
-        else { ep.residual_planes = in_p + r0 * d; ep.ldrp = d; ep.residual_plane_stride = M * d; }
-        ep.ln_gamma = w.ln1_gamma; ep.ln_beta = w.ln1_beta; ep.ln_eps = ln_eps;
-        ep.out_planes = h1_p + r0 * d; ep.ldpl = d; ep.plane_stride = M * d;
-        T4R_TRY(launch_gemm(pb, ep, sp));
-      }
-      // feed-forward (HF:xlnet:297-305): out = LN(h1 + gelu(h1 W1^T + b1) W2^T + b2)
-      {
-        GemmEpilogue ep;
-        ep.bias = w.b2;
-        ep.residual_planes = h1_p + r0 * d; ep.ldrp = d; ep.residual_plane_stride = M * d;
-        ep.ln_gamma = w.ln2_gamma; ep.ln_beta = w.ln2_beta; ep.ln_eps = ln_eps;
-        ep.out_f32 = dst_f ? dst_f + r0 * d : nullptr; ep.ldo = d;
-        ep.out_planes = dst_p ? dst_p + r0 * d : nullptr; ep.ldpl = d; ep.plane_stride = M * d;
-        if (use_ffn_fused(d)) {
-          T4R_TRY(launch_ffn_fused(h1_p + r0 * d, Mp, d, 4 * d, static_cast<const __nv_bfloat16*>(w.w1_planes), w.b1,
-                                   static_cast<const __nv_bfloat16*>(w.w2_planes), ep, sp, M * d));
-        } else {
-          {
-            GemmProblem pb;
-            pb.M = Mp; pb.N = 4 * d; pb.Kp = d;
-            pb.a_planes = h1_p + r0 * d; pb.a_rows = M;
-            pb.b_planes = static_cast<const __nv_bfloat16*>(w.w1_planes); pb.b_rows = 4 * d;
-            GemmEpilogue e1;
-            e1.bias = w.b1; e1.act = T4R_ACT_GELU;
-            e1.out_planes = ff_p + r0 * 4 * d; e1.ldpl = 4 * d; e1.plane_stride = M * 4 * d;
-            T4R_TRY(launch_gemm(pb, e1, sp));
-          }
-          GemmProblem pb;
-          pb.M = Mp; pb.N = d; pb.Kp = 4 * d;
-          pb.a_planes = ff_p + r0 * 4 * d; pb.a_rows = M;
-          pb.b_planes = static_cast<const __nv_bfloat16*>(w.w2_planes); pb.b_rows = d;
-          T4R_TRY(launch_gemm(pb, ep, sp));
-        }
-      }
+    // Q | K | V projections (HF:xlnet:253-259), one GEMM over the fused [3d, d] weight
+    {
+      GemmProblem pb;
+      pb.M = M; pb.N = 3 * d; pb.Kp = d;
+      pb.a_planes = in_p; pb.a_rows = M;
+      pb.b_planes = static_cast<const __nv_bfloat16*>(w.wqkv_planes); pb.b_rows = 3 * d;
+      GemmEpilogue ep;
+      if (tc_attn) { ep.out_planes = qkv_p; ep.ldpl = 3 * d; ep.plane_stride = M * 3 * d; }
+      else { ep.out_f32 = qkv; ep.ldo = 3 * d; }
+      T4R_TRY(launch_gemm(pb, ep, s));
+    }
+    // relative attention core (HF:xlnet:95-140)
+    if (plm_mask) {
+      T4R_REQUIRE(tc_attn, "xlnet_encoder_plm: the FFMA attention fallback has no two-stream form (unset T4R_ATTN_SIMT)");
+      T4R_TRY(launch_attn_mma_plm(qkv_p, M * 3 * d, r_p_l, static_cast<int64_t>(2) * L * d, w.r_w_bias, w.r_r_bias, B / 2,
+                                  L, d, n_head, attn_p, M * d, plm_mask, s));
+    } else if (tc_attn)
+      T4R_TRY(launch_attn_mma(true, qkv_p, M * 3 * d, r_p_l, static_cast<int64_t>(2) * L * d, w.r_w_bias, w.r_r_bias, B,
+                              L, d, n_head, attn_p, M * d, s));
+    else
+      T4R_TRY(launch_xlnet_attn(qkv, rbuf_l, w.r_w_bias, w.r_r_bias, B, L, d, n_head, attn_p, M * d, s));
+    // post_attention: h1 = LN(x + attn @ Wo^T) (HF:xlnet:142-152)
+    {
+      GemmProblem pb;
+      pb.M = M; pb.N = d; pb.Kp = d;
+      pb.a_planes = attn_p; pb.a_rows = M;
+      pb.b_planes = static_cast<const __nv_bfloat16*>(w.wo_planes); pb.b_rows = d;
+      GemmEpilogue ep;
+      // residual: the caller's fp32 x for the first layer, afterwards the split planes of the
+      // previous layer's output (hi + lo, exact to 16 mantissa bits) -- no fp32 copy of the
+      // residual stream is written between layers (the store path bounds these epilogues)
+      if (in_f) { ep.residual = in_f; ep.ldr = d; }
+      else { ep.residual_planes = in_p; ep.ldrp = d; ep.residual_plane_stride = M * d; }
+      ep.ln_gamma = w.ln1_gamma; ep.ln_beta = w.ln1_beta; ep.ln_eps = ln_eps;
+      ep.out_planes = h1_p; ep.ldpl = d; ep.plane_stride = M * d;
+      T4R_TRY(launch_gemm(pb, ep, s));
+    }
+    // feed-forward (HF:xlnet:297-305): out = LN(h1 + gelu(h1 W1^T + b1) W2^T + b2)
+    {
+      GemmEpilogue ep;
+      ep.bias = w.b2;
+      ep.residual_planes = h1_p; ep.ldrp = d; ep.residual_plane_stride = M * d;
+      ep.ln_gamma = w.ln2_gamma; ep.ln_beta = w.ln2_beta; ep.ln_eps = ln_eps;
+      ep.out_f32 = dst_f; ep.ldo = d;
+      ep.out_planes = dst_p; ep.ldpl = d; ep.plane_stride = M * d;
+      T4R_TRY(launch_ffn_fused(h1_p, M, d, 4 * d, static_cast<const __nv_bfloat16*>(w.w1_planes), w.b1,
+                               static_cast<const __nv_bfloat16*>(w.w2_planes), ep, s));
     }
     in_f = dst_f;
     in_p = dst_p;
-  }
-  if (nparts > 1) {
-    EncStreams* es = enc_streams();
-    for (int p = 1; p < nparts; ++p) {
-      T4R_CUDA(cudaEventRecord(es->join[p - 1], ps[p]));
-      T4R_CUDA(cudaStreamWaitEvent(s, es->join[p - 1], 0));
-    }
   }
   return 0;
 }
@@ -405,7 +305,6 @@ extern "C" size_t t4r_gpt2_encoder_workspace_bytes(int B, int L, int d, int n_he
   size_t b = 0;
   b += pad256(M * 3 * d * 4);      // qkv
   b += pad256(2 * M * d * 2);      // attention planes
-  b += pad256(2 * M * 4 * d * 2);  // ff planes
   b += 2 * pad256(M * d * 4);      // residual stream ping-pong
   b += 2 * pad256(2 * M * d * 2);  // LN output planes ping-pong
   return b + 1024;
@@ -424,7 +323,6 @@ extern "C" int t4r_gpt2_encoder_fwd(const t4r_gpt2_layer* layers, int n_layer, i
   Arena ar(workspace, workspace_bytes);
   float* qkv = ar.take<float>(M * 3 * d);
   __nv_bfloat16* attn_p = ar.take<__nv_bfloat16>(2 * M * d);
-  __nv_bfloat16* ff_p = ar.take<__nv_bfloat16>(2 * M * 4 * d);
   float* hbuf[2] = {ar.take<float>(M * d), ar.take<float>(M * d)};
   __nv_bfloat16* lnp[2] = {ar.take<__nv_bfloat16>(2 * M * d), ar.take<__nv_bfloat16>(2 * M * d)};
   T4R_REQUIRE(ar.ok, "gpt2_encoder: workspace carve-up failed");
@@ -483,26 +381,8 @@ extern "C" int t4r_gpt2_encoder_fwd(const t4r_gpt2_layer* layers, int n_layer, i
         ep.out_pre = hbuf[hc ^ 1]; ep.ldp = d;
         ep.out_planes = lnp[pc ^ 1]; ep.ldpl = d; ep.plane_stride = M * d;
       }
-      if (use_ffn_fused(d)) {
-        T4R_TRY(launch_ffn_fused(lnp[pc], M, d, 4 * d, static_cast<const __nv_bfloat16*>(w.w1_planes), w.b1,
-                                 static_cast<const __nv_bfloat16*>(w.w2_planes), ep, s));
-      } else {
-        {
-          GemmProblem pb;
-          pb.M = M; pb.N = 4 * d; pb.Kp = d;
-          pb.a_planes = lnp[pc]; pb.a_rows = M;
-          pb.b_planes = static_cast<const __nv_bfloat16*>(w.w1_planes); pb.b_rows = 4 * d;
-          GemmEpilogue e1;
-          e1.bias = w.b1; e1.act = T4R_ACT_GELU;
-          e1.out_planes = ff_p; e1.ldpl = 4 * d; e1.plane_stride = M * 4 * d;
-          T4R_TRY(launch_gemm(pb, e1, s));
-        }
-        GemmProblem pb;
-        pb.M = M; pb.N = d; pb.Kp = 4 * d;
-        pb.a_planes = ff_p; pb.a_rows = M;
-        pb.b_planes = static_cast<const __nv_bfloat16*>(w.w2_planes); pb.b_rows = d;
-        T4R_TRY(launch_gemm(pb, ep, s));
-      }
+      T4R_TRY(launch_ffn_fused(lnp[pc], M, d, 4 * d, static_cast<const __nv_bfloat16*>(w.w1_planes), w.b1,
+                               static_cast<const __nv_bfloat16*>(w.w2_planes), ep, s));
       hc ^= 1; pc ^= 1;
     }
   }

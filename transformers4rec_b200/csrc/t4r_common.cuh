@@ -28,22 +28,6 @@ __device__ __forceinline__ void mbar_init(uint64_t* bar, uint32_t count) {
 __device__ __forceinline__ void fence_barrier_init() {
   asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
 }
-// TMA store of a shared-memory box to global memory (bulk async group of the issuing thread)
-__device__ __forceinline__ void tma_store_2d(const void* tmap, const void* smem_src, int c0, int c1) {
-  asm volatile("cp.async.bulk.tensor.2d.global.shared::cta.bulk_group [%0, {%2, %3}], [%1];"
-               ::"l"(reinterpret_cast<uint64_t>(tmap)), "r"(smem_u32(smem_src)), "r"(c0), "r"(c1)
-               : "memory");
-}
-__device__ __forceinline__ void tma_store_commit() { asm volatile("cp.async.bulk.commit_group;" ::: "memory"); }
-// wait until at most N of this thread's bulk groups still READ their shared-memory source
-template <int N>
-__device__ __forceinline__ void tma_store_wait_read() {
-  asm volatile("cp.async.bulk.wait_group.read %0;" ::"n"(N) : "memory");
-}
-// generic-proxy writes (st.shared) -> visible to the async proxy (TMA / UMMA reads)
-__device__ __forceinline__ void fence_proxy_async_smem() {
-  asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
-}
 __device__ __forceinline__ void mbar_arrive_expect_tx(uint64_t* bar, uint32_t bytes) {
   asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(smem_u32(bar)), "r"(bytes)
                : "memory");
@@ -190,21 +174,6 @@ __device__ __forceinline__ uint64_t umma_desc_sw128(uint32_t smem_addr) {
   d |= static_cast<uint64_t>(1) << 46;
   d |= static_cast<uint64_t>(2) << 61;
   return d;
-}
-// Same for rows of 64 bytes with the 64-byte swizzle (TMA SWIZZLE_64B, 32 bf16 per row):
-// layout type 4, stride byte offset = 8 rows * 64 B = 512.
-__device__ __forceinline__ uint64_t umma_desc_sw64(uint32_t smem_addr) {
-  uint64_t d = 0;
-  d |= static_cast<uint64_t>((smem_addr >> 4) & 0x3FFFu);
-  d |= static_cast<uint64_t>(1) << 16;
-  d |= static_cast<uint64_t>(512 >> 4) << 32;
-  d |= static_cast<uint64_t>(1) << 46;
-  d |= static_cast<uint64_t>(4) << 61;
-  return d;
-}
-template <int RB>
-__device__ __forceinline__ uint64_t umma_desc(uint32_t smem_addr) {
-  return RB == 128 ? umma_desc_sw128(smem_addr) : umma_desc_sw64(smem_addr);
 }
 // Instruction descriptor, kind::f16: A,B = bf16 (format 1), D = f32 (format 1),
 // both operands K-major, M = 128, N = n.

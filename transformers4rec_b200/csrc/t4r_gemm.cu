@@ -19,7 +19,6 @@
 #include <math.h>
 #include <stdlib.h>
 #include <mutex>
-#include <type_traits>
 #include <unordered_map>
 
 #include "t4r_common.cuh"
@@ -47,43 +46,44 @@ static PFN_encodeTiled get_encode_fn() {
   return fn;
 }
 
-// Descriptors are pure functions of (base, rows, Kp, box_rows, rb): encoded once and kept (the same weights, the same
+// Descriptors are pure functions of (base, rows, Kp, box_rows): encoded once and kept (the same weights, the same
 // workspace slices and the same grow-only activation buffers come back every step; cuTensorMapEncodeTiled costs a
 // microsecond or two of host time per call and a GEMM launch needs four to six of them -- the launch-bound small
 // configurations spent a third of their host time here).  Bounded: the table is dropped when it reaches 8192 entries.
 struct TmapKey {
-  const void* base; int64_t rows; int Kp, box_rows, rb;
+  const void* base; int64_t rows; int Kp, box_rows;
   bool operator==(const TmapKey& o) const {
-    return base == o.base && rows == o.rows && Kp == o.Kp && box_rows == o.box_rows && rb == o.rb;
+    return base == o.base && rows == o.rows && Kp == o.Kp && box_rows == o.box_rows;
   }
 };
 struct TmapKeyHash {
   size_t operator()(const TmapKey& k) const {
     uint64_t h = reinterpret_cast<uintptr_t>(k.base) * 0x9E3779B97F4A7C15ull;
     h ^= static_cast<uint64_t>(k.rows) * 0xC2B2AE3D27D4EB4Full + (static_cast<uint64_t>(k.Kp) << 20) +
-         (static_cast<uint64_t>(k.box_rows) << 8) + static_cast<uint64_t>(k.rb);
+         (static_cast<uint64_t>(k.box_rows) << 8);
     return static_cast<size_t>(h ^ (h >> 29));
   }
 };
 static std::mutex g_tmap_mu;
 static std::unordered_map<TmapKey, CUtensorMap, TmapKeyHash> g_tmap_cache;
 
-static int make_tmap_uncached(CUtensorMap* map, const __nv_bfloat16* base, int64_t rows, int Kp, int box_rows, int rb);
-static int make_tmap(CUtensorMap* map, const __nv_bfloat16* base, int64_t rows, int Kp, int box_rows, int rb) {
-  const TmapKey key{base, rows, Kp, box_rows, rb};
+static int make_tmap_uncached(CUtensorMap* map, const __nv_bfloat16* base, int64_t rows, int Kp, int box_rows);
+static int make_tmap(CUtensorMap* map, const __nv_bfloat16* base, int64_t rows, int Kp, int box_rows) {
+  const TmapKey key{base, rows, Kp, box_rows};
   {
     std::lock_guard<std::mutex> lk(g_tmap_mu);
     auto it = g_tmap_cache.find(key);
     if (it != g_tmap_cache.end()) { *map = it->second; return 0; }
   }
-  T4R_TRY(make_tmap_uncached(map, base, rows, Kp, box_rows, rb));
+  T4R_TRY(make_tmap_uncached(map, base, rows, Kp, box_rows));
   std::lock_guard<std::mutex> lk(g_tmap_mu);
   if (g_tmap_cache.size() >= 8192) g_tmap_cache.clear();
   g_tmap_cache.emplace(key, *map);
   return 0;
 }
 
-static int make_tmap_uncached(CUtensorMap* map, const __nv_bfloat16* base, int64_t rows, int Kp, int box_rows, int rb) {
+// box = 64 bf16 (128 bytes) of K x box_rows rows, 128-byte swizzle
+static int make_tmap_uncached(CUtensorMap* map, const __nv_bfloat16* base, int64_t rows, int Kp, int box_rows) {
   PFN_encodeTiled fn = get_encode_fn();
   if (!fn) {
     set_error("cuTensorMapEncodeTiled entry point not available (no CUDA driver?)");
@@ -95,11 +95,10 @@ static int make_tmap_uncached(CUtensorMap* map, const __nv_bfloat16* base, int64
   }
   cuuint64_t gdim[2] = {static_cast<cuuint64_t>(Kp), static_cast<cuuint64_t>(rows)};
   cuuint64_t gstride[1] = {static_cast<cuuint64_t>(Kp) * 2};
-  cuuint32_t box[2] = {static_cast<cuuint32_t>(rb / 2), static_cast<cuuint32_t>(box_rows)};
+  cuuint32_t box[2] = {64u, static_cast<cuuint32_t>(box_rows)};
   cuuint32_t estr[2] = {1u, 1u};
   CUresult r = fn(map, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 2, const_cast<__nv_bfloat16*>(base), gdim, gstride, box, estr,
-                  CU_TENSOR_MAP_INTERLEAVE_NONE, rb == 128 ? CU_TENSOR_MAP_SWIZZLE_128B : CU_TENSOR_MAP_SWIZZLE_64B,
-                  CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
+                  CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
                   CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
   if (r != CUDA_SUCCESS) {
     set_error("cuTensorMapEncodeTiled failed (CUresult %d) rows=%lld Kp=%d box_rows=%d", (int)r, (long long)rows, Kp,
@@ -109,23 +108,14 @@ static int make_tmap_uncached(CUtensorMap* map, const __nv_bfloat16* base, int64
   return 0;
 }
 
-int make_tmap_public(CUtensorMap* map, const __nv_bfloat16* base, int64_t rows, int Kp, int box_rows, int rb) {
-  return make_tmap(map, base, rows, Kp, box_rows, rb);
+int make_tmap_public(CUtensorMap* map, const __nv_bfloat16* base, int64_t rows, int Kp, int box_rows) {
+  return make_tmap(map, base, rows, Kp, box_rows);
 }
 
 // ----------------------------------------------------------------------------
 // kernel
 // ----------------------------------------------------------------------------
 constexpr int BM = 128;
-#ifndef T4R_GEMM_TMA_STORE_DEFAULT
-#define T4R_GEMM_TMA_STORE_DEFAULT 0
-#endif
-#ifndef T4R_FFN_EPW_DEFAULT
-#define T4R_FFN_EPW_DEFAULT 8
-#endif
-#ifndef T4R_FFN_2CTA_DEFAULT
-#define T4R_FFN_2CTA_DEFAULT 0
-#endif
 #ifndef T4R_HEAD_RESIDENT_DEFAULT
 #define T4R_HEAD_RESIDENT_DEFAULT 1  // resident-A head kernel (validated on B200 in round 2; T4R_HEAD_RESIDENT=0 selects the streaming CTA-pair kernel)
 #endif
@@ -133,17 +123,14 @@ constexpr int BM = 128;
 #define T4R_GEMM_2CTA_DEFAULT 1
 #endif
 
-// RB = bytes per shared-memory operand row = K extent of one pipeline stage (RB/2 bf16).
-// RB = 64 (SWIZZLE_64B) halves the stage and doubles the ring depth in the same shared memory
-// (4 stages of look-ahead instead of 2 at BN = 256).  Both variants are kept: they measure the
-// same on B200, see launch_gemm.
-template <int BN, int RB>
+// One pipeline stage holds 64 bf16 of K: shared-memory operand rows of 128 bytes.
+template <int BN>
 struct GemmCfg {
-  static constexpr int A_PLANE_BYTES = BM * RB;
-  static constexpr int B_PLANE_BYTES = BN * RB;
+  static constexpr int A_PLANE_BYTES = BM * 128;
+  static constexpr int B_PLANE_BYTES = BN * 128;
   static constexpr int STAGE_BYTES = 2 * A_PLANE_BYTES + 2 * B_PLANE_BYTES;
-  static constexpr int STAGES = (RB == 64) ? 4 : ((BN == 256) ? 2 : ((BN == 128) ? 3 : 4));
-  static constexpr int KSTEPS = RB / 32;   // UMMA K = 16 bf16 = 32 bytes
+  static constexpr int STAGES = (BN == 256) ? 2 : ((BN == 128) ? 3 : 4);
+  static constexpr int KSTEPS = 4;   // UMMA K = 16 bf16 = 32 bytes
   static constexpr int TMEM_COLS = 2 * BN;  // two accumulator stages (power of two)
   static constexpr int SMEM_BYTES = STAGES * STAGE_BYTES + 1024 /*align*/ + 256 /*barriers*/ + 4096 /*LN exchange*/ + 8 * 32 * 20 * 4 /*epilogue staging*/;
 };
@@ -421,16 +408,12 @@ __device__ __forceinline__ void residual_add(const GemmEpilogue& ep, float* stg_
   }
 }
 
-// NG = column groups a tile's row is split into (one epilogue warp per TMEM lane quadrant and group: 4 NG epilogue warps
-// per CTA).  NG = 2 is the original eight-warp form (bit-identical); NG = 4 halves every warp's share of the latency-
-// bound work (staging transposes, residual loads, stores) with twice the warps in flight.  With NG > 2 the residual
-// prefetch of the next chunk is dropped (registers: 576 threads leave 112 per thread) -- thread-level parallelism hides
-// that latency instead.  xch_grp0 = this row's slot in group 0 of the exchange area [NG][128]; grp = own group.
-template <int BN, int NG>
+// A tile's row is split into two column groups (warps 2-5 and 6-9).  xch_grp0 = this row's slot in group 0 of the
+// exchange area [2][128]; grp = own group.
+template <int BN>
 __device__ __forceinline__ void epilogue_ln_chunked(const GemmDev& p, uint32_t taddr, int64_t row0, int rows_valid, int lane,
                                                     int64_t n0, float* stg, float2* xch_grp0, int grp) {
-  constexpr int COLS = BN / NG, NCH = COLS / 32;
-  constexpr bool PREFETCH = (NG == 2);
+  constexpr int COLS = BN / 2, NCH = COLS / 32;
   const GemmEpilogue& ep = p.ep;
   if (ep.debug & 1) rows_valid = 0;
   const bool row_ok = lane < rows_valid;
@@ -441,19 +424,15 @@ __device__ __forceinline__ void epilogue_ln_chunked(const GemmDev& p, uint32_t t
   const bool lprof = (ep.debug & 2) && blockIdx.x == 0 && threadIdx.x == 64;
   const long long l0 = lprof ? clock64() : 0;
   // ---- pass 1: bias (+act, mask) + residual, statistics, park the pre-LN values in TMEM
-  uint4 nxt[PREFETCH ? 8 : 1];
-  if (PREFETCH && has_res) residual_issue(ep, row0, n0, rows_valid, lane, *reinterpret_cast<uint4(*)[8]>(nxt));
+  uint4 nxt[8];
+  if (has_res) residual_issue(ep, row0, n0, rows_valid, lane, nxt);
   float mean_h = 0.f, m2_h = 0.f;
 #pragma unroll
   for (int c = 0; c < NCH; ++c) {
     uint4 cur[8];
-    if constexpr (PREFETCH) {
 #pragma unroll
-      for (int j = 0; j < 8; ++j) cur[j] = nxt[j];
-      if (has_res && c + 1 < NCH) residual_issue(ep, row0, n0 + (c + 1) * 32, rows_valid, lane, *reinterpret_cast<uint4(*)[8]>(nxt));
-    } else {
-      if (has_res) residual_issue(ep, row0, n0 + c * 32, rows_valid, lane, cur);
-    }
+    for (int j = 0; j < 8; ++j) cur[j] = nxt[j];
+    if (has_res && c + 1 < NCH) residual_issue(ep, row0, n0 + (c + 1) * 32, rows_valid, lane, nxt);
     float v[32];
     tmem_ld<32>(taddr + c * 32, v);
     dense_chunk(v, ep, n0 + c * 32, code);
@@ -476,25 +455,13 @@ __device__ __forceinline__ void epilogue_ln_chunked(const GemmDev& p, uint32_t t
   }
   tmem_st_wait();
   const long long l1 = lprof ? clock64() : 0;
-  // ---- combine the NG groups of the row (equal counts)
+  // ---- combine the two groups of the row (equal counts)
   xch_grp0[grp * 128] = make_float2(mean_h, m2_h);
-  asm volatile("bar.sync 1, %0;" ::"n"(NG * 128) : "memory");
-  float mean, m2;
-  if constexpr (NG == 2) {
-    const float2 o = xch_grp0[(grp ^ 1) * 128];
-    const float delta = o.x - mean_h;
-    mean = 0.5f * (mean_h + o.x);
-    m2 = m2_h + o.y + delta * delta * (0.5f * COLS);
-  } else {
-    float2 part[NG];
-    float sum = 0.f;
-#pragma unroll
-    for (int g = 0; g < NG; ++g) { part[g] = xch_grp0[g * 128]; sum += part[g].x; }
-    mean = sum * (1.f / NG);
-    m2 = 0.f;
-#pragma unroll
-    for (int g = 0; g < NG; ++g) { const float dl = part[g].x - mean; m2 += part[g].y + dl * dl * static_cast<float>(COLS); }
-  }
+  asm volatile("bar.sync 1, %0;" ::"n"(2 * 128) : "memory");
+  const float2 o = xch_grp0[(grp ^ 1) * 128];
+  const float delta = o.x - mean_h;
+  const float mean = 0.5f * (mean_h + o.x);
+  const float m2 = m2_h + o.y + delta * delta * (0.5f * COLS);
   const float rstd = rsqrtf(m2 * (1.f / BN) + ep.ln_eps);
   const long long l2 = lprof ? clock64() : 0;
   // ---- pass 2: normalise and store
@@ -526,10 +493,10 @@ __device__ __forceinline__ void epilogue_ln_chunked(const GemmDev& p, uint32_t t
 // Each epilogue thread owns one output row (its TMEM lane) and COLS = BN/2 columns
 // (warps 2-5 take the first half of the tile's columns, warps 6-9 the second half).
 // row0 = first row of the warp's 32-row block; n0 = first column of the warp's half.
-template <int BN, bool LN, int NG = 2>
+template <int BN, bool LN>
 __device__ __forceinline__ void epilogue_dense(const GemmDev& p, uint32_t taddr, int64_t row0, int rows_valid, int lane,
                                                int64_t n0, float* stg, float2* xch_grp0, int grp) {
-  constexpr int COLS = BN / NG;
+  constexpr int COLS = BN / 2;
   const GemmEpilogue& ep = p.ep;
   if (ep.debug & 1) rows_valid = 0;  // timing experiment: no global traffic from the epilogue
   const bool row_ok = lane < rows_valid;
@@ -537,7 +504,7 @@ __device__ __forceinline__ void epilogue_dense(const GemmDev& p, uint32_t taddr,
   int code = 0;
   if (row_ok && ep.row_code) code = ep.row_code[row];
   if constexpr (LN) {
-    epilogue_ln_chunked<BN, NG>(p, taddr, row0, rows_valid, lane, n0, stg, xch_grp0, grp);
+    epilogue_ln_chunked<BN>(p, taddr, row0, rows_valid, lane, n0, stg, xch_grp0, grp);
   } else {
     const bool prof = (ep.debug & 2) && blockIdx.x == 0 && threadIdx.x == 64;
 #pragma unroll 1
@@ -582,53 +549,6 @@ __device__ __forceinline__ void epilogue_dense(const GemmDev& p, uint32_t taddr,
         warp_store_planes(stg, v, ep.out_planes + row0 * ep.ldpl + ncol0, ep.plane_stride, ep.ldpl, rows_valid, lane);
       if (prof) { long long t4 = clock64(); g_dbg_cycles[4] += t3 - t2; g_dbg_cycles[5] += t4 - t3; }
     }
-  }
-}
-
-// Dense epilogue with TMA STORES (planes-only outputs, no residual / LayerNorm / mask: the Q|K|V projection, whose
-// 126 MB of plane stores per call bound it).  Each thread splits its row's 32-column chunk to bf16 hi / lo and writes
-// the two 64-byte row pieces into a 64B-swizzled [32 rows x 64 B] shared-memory box per plane (16-byte chunk j of row
-// r sits at chunk j ^ ((r >> 1) & 3): the layout CU_TENSOR_MAP_SWIZZLE_64B expects, and conflict-free for one row per
-// lane); one lane then issues two cp.async.bulk.tensor stores.  No row <-> column transposition through a staging
-// tile, no per-lane global store instructions, and the stores drain asynchronously while the next chunk is computed
-// (two boxes per warp, `cp.async.bulk.wait_group.read 1` before a box is rewritten).  Rows / columns outside the
-// tensor are clipped by the TMA unit.
-template <int BN>
-__device__ __forceinline__ void epilogue_dense_tma(const GemmDev& p, uint32_t taddr, int64_t row0, int lane, int64_t n0,
-                                                   uint8_t* boxes, uint32_t& nstores, const CUtensorMap* tm_hi,
-                                                   const CUtensorMap* tm_lo) {
-  constexpr int COLS = BN / 2;
-  const GemmEpilogue& ep = p.ep;
-  const int sw = (lane >> 1) & 3;
-#pragma unroll 1
-  for (int c = 0; c < COLS / 32; ++c) {
-    float v[32];
-    tmem_ld<32>(taddr + c * 32, v);
-    const int64_t ncol0 = n0 + c * 32;
-    if (ncol0 >= p.N) continue;   // warp-uniform
-    dense_chunk(v, ep, ncol0, 0);
-    uint32_t h[16], l[16];
-#pragma unroll
-    for (int j = 0; j < 16; ++j) split_bf16x2(v[2 * j], v[2 * j + 1], h[j], l[j]);
-    uint8_t* box = boxes + (nstores & 1u) * 4096u;
-    if (nstores >= 2) {
-      if (lane == 0) tma_store_wait_read<1>();   // the stores issued from this box two chunks ago have read it
-      __syncwarp();
-    }
-#pragma unroll
-    for (int j = 0; j < 4; ++j) {
-      const int off = lane * 64 + ((j ^ sw) << 4);
-      *reinterpret_cast<uint4*>(box + off) = make_uint4(h[4 * j], h[4 * j + 1], h[4 * j + 2], h[4 * j + 3]);
-      *reinterpret_cast<uint4*>(box + 2048 + off) = make_uint4(l[4 * j], l[4 * j + 1], l[4 * j + 2], l[4 * j + 3]);
-    }
-    fence_proxy_async_smem();
-    __syncwarp();
-    if (lane == 0) {
-      tma_store_2d(tm_hi, box, static_cast<int>(ncol0), static_cast<int>(row0));
-      tma_store_2d(tm_lo, box + 2048, static_cast<int>(ncol0), static_cast<int>(row0));
-      tma_store_commit();
-    }
-    ++nstores;
   }
 }
 
@@ -756,12 +676,12 @@ __device__ __forceinline__ void epilogue_head(const GemmDev& p, uint32_t taddr, 
   }
 }
 
-template <int BN, bool LN, bool HEAD, int RB>
+template <int BN, bool LN, bool HEAD>
 __global__ void __launch_bounds__(320, 1)
 gemm_bf16x3_kernel(const __grid_constant__ CUtensorMap tmAh, const __grid_constant__ CUtensorMap tmAl,
                    const __grid_constant__ CUtensorMap tmBh, const __grid_constant__ CUtensorMap tmBl,
                    const GemmDev p) {
-  using Cfg = GemmCfg<BN, RB>;
+  using Cfg = GemmCfg<BN>;
   constexpr int A_PLANE_BYTES = Cfg::A_PLANE_BYTES;
   extern __shared__ uint8_t smem_raw[];
   // 1024-byte alignment for the 128B-swizzled tiles, done with pointer arithmetic on the
@@ -823,12 +743,11 @@ gemm_bf16x3_kernel(const __grid_constant__ CUtensorMap tmAh, const __grid_consta
           mbar_wait(&empty_bar[stage], phase ^ 1);
           uint8_t* st = smem + stage * Cfg::STAGE_BYTES;
           mbar_arrive_expect_tx(&full_bar[stage], bytes);
-          constexpr int KE = RB / 2;  // bf16 elements of K per stage
-          tma_load_2d(st, &tmAh, &full_bar[stage], kb * KE, m0);
-          tma_load_2d(st + 2 * A_PLANE_BYTES, &tmBh, &full_bar[stage], kb * KE, n0);
+          tma_load_2d(st, &tmAh, &full_bar[stage], kb * 64, m0);
+          tma_load_2d(st + 2 * A_PLANE_BYTES, &tmBh, &full_bar[stage], kb * 64, n0);
           if (p.nprod != 1) {
-            tma_load_2d(st + A_PLANE_BYTES, &tmAl, &full_bar[stage], kb * KE, m0);
-            tma_load_2d(st + 2 * A_PLANE_BYTES + Cfg::B_PLANE_BYTES, &tmBl, &full_bar[stage], kb * KE, n0);
+            tma_load_2d(st + A_PLANE_BYTES, &tmAl, &full_bar[stage], kb * 64, m0);
+            tma_load_2d(st + 2 * A_PLANE_BYTES + Cfg::B_PLANE_BYTES, &tmBl, &full_bar[stage], kb * 64, n0);
           }
           if (++stage == Cfg::STAGES) { stage = 0; phase ^= 1; }
         }
@@ -854,7 +773,7 @@ gemm_bf16x3_kernel(const __grid_constant__ CUtensorMap tmAh, const __grid_consta
           const uint32_t a_lo = a_hi + A_PLANE_BYTES;
           const uint32_t b_hi = a_hi + 2 * A_PLANE_BYTES;
           const uint32_t b_lo = b_hi + Cfg::B_PLANE_BYTES;
-          if (RB == 128 && p.nprod == 2) {
+          if (p.nprod == 2) {
             // 2-unit product (t4r_mixed_pack.cuh): plane 0 = fp16, plane 1 = [64 x hi8 | 64 x lo8] e4m3 per row.
             // Four K = 16 fp16 MMAs, then lo8(A) x hi8(B) and hi8(A) x lo8(B) as two K = 32 e4m3 MMAs each,
             // all into the same fp32 accumulator.
@@ -866,23 +785,23 @@ gemm_bf16x3_kernel(const __grid_constant__ CUtensorMap tmAh, const __grid_consta
             if (!(dbg & 64)) {
 #pragma unroll
               for (int k4 = 0; k4 < 4; ++k4) {
-                umma_bf16(d_tmem, umma_desc<RB>(a_hi + k4 * 32), umma_desc<RB>(b_hi + k4 * 32), idesc_h, acc);
+                umma_bf16(d_tmem, umma_desc_sw128(a_hi + k4 * 32), umma_desc_sw128(b_hi + k4 * 32), idesc_h, acc);
                 acc = 1u;
               }
             }
 #pragma unroll
             for (int j = 0; j < 2; ++j) {
-              if (!(dbg & 128)) { umma_f8(d_tmem, umma_desc<RB>(a_lo + 64 + j * 32), umma_desc<RB>(b_lo + j * 32), idesc_8, acc); acc = 1u; }
-              if (!(dbg & 256)) { umma_f8(d_tmem, umma_desc<RB>(a_lo + j * 32), umma_desc<RB>(b_lo + 64 + j * 32), idesc_8, acc); acc = 1u; }
+              if (!(dbg & 128)) { umma_f8(d_tmem, umma_desc_sw128(a_lo + 64 + j * 32), umma_desc_sw128(b_lo + j * 32), idesc_8, acc); acc = 1u; }
+              if (!(dbg & 256)) { umma_f8(d_tmem, umma_desc_sw128(a_lo + j * 32), umma_desc_sw128(b_lo + 64 + j * 32), idesc_8, acc); acc = 1u; }
             }
           } else {
 #pragma unroll
           for (int k4 = 0; k4 < Cfg::KSTEPS; ++k4) {
-            const uint64_t da_hi = umma_desc<RB>(a_hi + k4 * 32);
-            const uint64_t db_hi = umma_desc<RB>(b_hi + k4 * 32);
+            const uint64_t da_hi = umma_desc_sw128(a_hi + k4 * 32);
+            const uint64_t db_hi = umma_desc_sw128(b_hi + k4 * 32);
             if (p.nprod == 3) {
-              const uint64_t da_lo = umma_desc<RB>(a_lo + k4 * 32);
-              const uint64_t db_lo = umma_desc<RB>(b_lo + k4 * 32);
+              const uint64_t da_lo = umma_desc_sw128(a_lo + k4 * 32);
+              const uint64_t db_lo = umma_desc_sw128(b_lo + k4 * 32);
               umma_bf16(d_tmem, da_lo, db_hi, idesc, (kb | k4) != 0);
               umma_bf16(d_tmem, da_hi, db_lo, idesc, 1u);
               umma_bf16(d_tmem, da_hi, db_hi, idesc, 1u);
@@ -967,26 +886,12 @@ struct Gemm2Cfg {
   static constexpr int SMEM_BYTES = STAGES * STAGE_BYTES + 1024 + 256 + 4096 + 8 * 32 * 20 * 4;
 };
 
-// TMA-store variant of the configuration: two ring stages (these GEMMs are epilogue-bound) and, instead of the
-// per-warp staging tiles, two 4 KB store boxes per epilogue warp (1024-byte aligned).
-template <int BN>
-struct Gemm2CfgTma {
-  static constexpr int A_PLANE_BYTES = Gemm2Cfg<BN>::A_PLANE_BYTES;
-  static constexpr int B_PLANE_BYTES = Gemm2Cfg<BN>::B_PLANE_BYTES;
-  static constexpr int STAGE_BYTES = Gemm2Cfg<BN>::STAGE_BYTES;
-  static constexpr int STAGES = 2;
-  static constexpr int TMEM_COLS = 2 * BN;
-  static constexpr int BOX_BYTES = 8 * 2 * 4096;
-  static constexpr int SMEM_BYTES = STAGES * STAGE_BYTES + 1024 /*align*/ + 1024 /*barriers, keeps the boxes aligned*/ + BOX_BYTES;
-};
-
-template <int BN, bool LN, bool HEAD, bool TMAOUT = false>
+template <int BN, bool LN, bool HEAD>
 __global__ void __launch_bounds__(320, 1)
 gemm2_bf16x3_kernel(const __grid_constant__ CUtensorMap tmAh, const __grid_constant__ CUtensorMap tmAl,
                     const __grid_constant__ CUtensorMap tmBh, const __grid_constant__ CUtensorMap tmBl,
-                    const __grid_constant__ CUtensorMap tmOh, const __grid_constant__ CUtensorMap tmOl,
                     const GemmDev p) {
-  using Cfg = typename std::conditional<TMAOUT, Gemm2CfgTma<BN>, Gemm2Cfg<BN>>::type;
+  using Cfg = Gemm2Cfg<BN>;
   constexpr int A_PLANE_BYTES = Cfg::A_PLANE_BYTES;
   extern __shared__ uint8_t smem_raw[];
   uint8_t* smem = smem_raw + ((1024u - (smem_u32(smem_raw) & 1023u)) & 1023u);
@@ -997,7 +902,6 @@ gemm2_bf16x3_kernel(const __grid_constant__ CUtensorMap tmAh, const __grid_const
   uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(tempty_bar + 2);
   float2* xch = reinterpret_cast<float2*>(smem + Cfg::STAGES * Cfg::STAGE_BYTES + 256);
   float* stg_all = reinterpret_cast<float*>(smem + Cfg::STAGES * Cfg::STAGE_BYTES + 256 + 4096);
-  uint8_t* box_all = smem + Cfg::STAGES * Cfg::STAGE_BYTES + 1024;   // TMAOUT: [8 warps][2 boxes][hi 2 KB | lo 2 KB]
 
   const int warp = warp_id();
   const int lane = lane_id();
@@ -1129,7 +1033,6 @@ gemm2_bf16x3_kernel(const __grid_constant__ CUtensorMap tmAh, const __grid_const
     int as = 0;
     uint32_t aph = 0;
     uint32_t tile_parity = 0;
-    uint32_t nstores = 0;   // TMAOUT: chunks this warp has handed to the TMA unit (selects the box, paces its reuse)
     for (int64_t tile = pair; tile < num_tiles; tile += npairs) {
       const int tile_n = static_cast<int>(tile / tiles_m);
       const int64_t m0 = static_cast<int64_t>(tile % tiles_m) * (2 * BM) + rank * BM;
@@ -1143,9 +1046,6 @@ gemm2_bf16x3_kernel(const __grid_constant__ CUtensorMap tmAh, const __grid_const
       const bool row_ok = row < M_eff;
       if (HEAD) {
         epilogue_head<BN>(p, taddr, row, row_ok, n0, tile_n * 2 + half);
-      } else if constexpr (TMAOUT) {
-        if (row0 < M_eff)   // warp-uniform; a block of rows wholly beyond M is not stored (partial blocks: TMA clips)
-          epilogue_dense_tma<BN>(p, taddr, row0, lane, n0, box_all + (warp - 2) * 8192, nstores, &tmOh, &tmOl);
       } else {
         float2* xg0 = xch + (tile_parity * 2) * 128 + quad * 32 + lane;   // [parity][group][row]
         const int64_t left = static_cast<int64_t>(M_eff) - row0;
@@ -1161,9 +1061,6 @@ gemm2_bf16x3_kernel(const __grid_constant__ CUtensorMap tmAh, const __grid_const
     }
   }
 
-  if constexpr (TMAOUT) {
-    if (warp >= 2 && lane == 0) tma_store_wait_read<0>();   // shared memory must outlive the stores that read it
-  }
   tc_fence_before_sync();
   __syncthreads();
   cluster_sync_all();  // no CTA tears down its barriers / TMEM while the peer may still signal or read them
@@ -1604,11 +1501,11 @@ static int num_sms() {
   return g_num_sms;
 }
 
-template <int BN, bool LN, bool HEAD, int RB>
+template <int BN, bool LN, bool HEAD>
 static int launch_inst(const CUtensorMap& ah, const CUtensorMap& al, const CUtensorMap& bh, const CUtensorMap& bl,
                        const GemmDev& dp, int64_t max_tiles, cudaStream_t stream) {
-  using Cfg = GemmCfg<BN, RB>;
-  auto kern = gemm_bf16x3_kernel<BN, LN, HEAD, RB>;
+  using Cfg = GemmCfg<BN>;
+  auto kern = gemm_bf16x3_kernel<BN, LN, HEAD>;
   static bool attr_set = false;
   if (!attr_set) {
     T4R_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, Cfg::SMEM_BYTES));
@@ -1622,14 +1519,11 @@ static int launch_inst(const CUtensorMap& ah, const CUtensorMap& al, const CUten
 }
 
 
-template <int BN, bool LN, bool HEAD, bool TMAOUT = false>
+template <int BN, bool LN, bool HEAD>
 static int launch_inst2(const CUtensorMap& ah, const CUtensorMap& al, const CUtensorMap& bh, const CUtensorMap& bl,
-                        const GemmDev& dp, int64_t max_pair_tiles, cudaStream_t stream,
-                        const CUtensorMap* oh = nullptr, const CUtensorMap* ol = nullptr) {
-  using Cfg = typename std::conditional<TMAOUT, Gemm2CfgTma<BN>, Gemm2Cfg<BN>>::type;
-  auto kern = gemm2_bf16x3_kernel<BN, LN, HEAD, TMAOUT>;
-  const CUtensorMap& toh = oh ? *oh : ah;   // unused unless TMAOUT
-  const CUtensorMap& tol = ol ? *ol : al;
+                        const GemmDev& dp, int64_t max_pair_tiles, cudaStream_t stream) {
+  using Cfg = Gemm2Cfg<BN>;
+  auto kern = gemm2_bf16x3_kernel<BN, LN, HEAD>;
   static bool attr_set = false;
   if (!attr_set) {
     T4R_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, Cfg::SMEM_BYTES));
@@ -1650,7 +1544,7 @@ static int launch_inst2(const CUtensorMap& ah, const CUtensorMap& al, const CUte
   attr[0].val.clusterDim.z = 1;
   cfg.attrs = attr;
   cfg.numAttrs = 1;
-  T4R_CUDA(cudaLaunchKernelEx(&cfg, kern, ah, al, bh, bl, toh, tol, dp));
+  T4R_CUDA(cudaLaunchKernelEx(&cfg, kern, ah, al, bh, bl, dp));
   T4R_LAUNCH_CHECK("gemm2_bf16x3_kernel");
   return 0;
 }
@@ -1696,16 +1590,14 @@ extern "C" int t4r_debug_gemm_cycles(unsigned long long* out8, int reset) {
 }
 namespace t4r {
 // T4R_HEAD_RESIDENT != 0 (the default) and a shape the resident-A head kernel covers: K <= 256, more than one 128-row
-// block, CTA pairs and 128-byte rows enabled.  Returns the number of LSE partials per row the head call must size
+// block, CTA pairs enabled.  Returns the number of LSE partials per row the head call must size
 // for (2 per column CHUNK), or 0 when the regular kernels run (2 per column TILE).
 int head_resident_partials(int64_t M, int64_t V, int Kp) {
   int resident = T4R_HEAD_RESIDENT_DEFAULT;
   if (const char* e = getenv("T4R_HEAD_RESIDENT")) resident = atoi(e);
   int two_cta = T4R_GEMM_2CTA_DEFAULT;
   if (const char* e = getenv("T4R_GEMM_2CTA")) two_cta = atoi(e);
-  const char* rbe = getenv("T4R_GEMM_RB");
-  const bool rb128 = !(rbe && atoi(rbe) == 64);
-  if (!resident || !two_cta || !rb128 || M <= BM || Kp > 64 * HeadResCfg::MAX_KB) return 0;
+  if (!resident || !two_cta || M <= BM || Kp > 64 * HeadResCfg::MAX_KB) return 0;
   const int64_t tiles_n = (V + HeadResCfg::BN - 1) / HeadResCfg::BN;
   const int hc = head_chunk();
   return 2 * static_cast<int>((tiles_n + hc - 1) / hc);
@@ -1736,22 +1628,16 @@ int launch_gemm(const GemmProblem& pb, const GemmEpilogue& ep, cudaStream_t stre
   }
   T4R_REQUIRE(bn == 64 || bn == 128 || bn == 256, "gemm: bad BN %d", bn);
 
-  // Row width of the shared-memory operand tiles.  Default 128 B (2 x 96 KB stages at BN = 256);
-  // T4R_GEMM_RB=64 selects 64-byte rows (4 x 48 KB stages).  Measured equal on B200 (head GEMM
-  // 4.98 ms vs 5.15 ms): the kernel runs at the power-capped tensor rate, not on TMA latency.
-  static int rb = 0;
-  if (rb == 0) { const char* e = getenv("T4R_GEMM_RB"); rb = (e && atoi(e) == 64) ? 64 : 128; }
-  T4R_REQUIRE(pb.nprod != 2 || rb == 128, "gemm: nprod = 2 needs 128-byte operand rows (unset T4R_GEMM_RB)");
   CUtensorMap ah, al, bh, bl;
-  T4R_TRY(make_tmap(&ah, pb.a_planes, pb.M, pb.Kp, BM, rb));
-  T4R_TRY(make_tmap(&al, pb.a_planes + pb.a_rows * pb.Kp, pb.M, pb.Kp, BM, rb));
-  T4R_TRY(make_tmap(&bh, pb.b_planes, pb.N, pb.Kp, bn, rb));
-  T4R_TRY(make_tmap(&bl, pb.b_planes + pb.b_rows * pb.Kp, pb.N, pb.Kp, bn, rb));
+  T4R_TRY(make_tmap(&ah, pb.a_planes, pb.M, pb.Kp, BM));
+  T4R_TRY(make_tmap(&al, pb.a_planes + pb.a_rows * pb.Kp, pb.M, pb.Kp, BM));
+  T4R_TRY(make_tmap(&bh, pb.b_planes, pb.N, pb.Kp, bn));
+  T4R_TRY(make_tmap(&bl, pb.b_planes + pb.b_rows * pb.Kp, pb.N, pb.Kp, bn));
 
   GemmDev dp;
   dp.M = static_cast<int>(pb.M);
   dp.N = pb.N;
-  dp.nkb = pb.Kp / (rb / 2);
+  dp.nkb = pb.Kp / 64;
   dp.nprod = pb.nprod;
   dp.head_chunk = head_chunk();
   dp.m_dev = pb.m_dev;
@@ -1762,13 +1648,13 @@ int launch_gemm(const GemmProblem& pb, const GemmEpilogue& ep, cudaStream_t stre
   }
   const int64_t max_tiles = ((pb.M + BM - 1) / BM) * ((pb.N + bn - 1) / bn);
 
-  // T4R_GEMM_2CTA=1: CTA-pair kernel (cta_group::2, 256-row tiles).  Needs 128-byte rows and more than one 128-row tile.
+  // T4R_GEMM_2CTA=1: CTA-pair kernel (cta_group::2, 256-row tiles).  Needs more than one 128-row tile.
   int two_cta = T4R_GEMM_2CTA_DEFAULT;  // read per call so that tests can exercise both kernels in one process
   if (const char* e = getenv("T4R_GEMM_2CTA")) two_cta = atoi(e);
-  if (two_cta && rb == 128 && pb.M > BM) {
+  if (two_cta && pb.M > BM) {
     CUtensorMap bh2, bl2;
-    T4R_TRY(make_tmap(&bh2, pb.b_planes, pb.N, pb.Kp, bn / 2, rb));
-    T4R_TRY(make_tmap(&bl2, pb.b_planes + pb.b_rows * pb.Kp, pb.N, pb.Kp, bn / 2, rb));
+    T4R_TRY(make_tmap(&bh2, pb.b_planes, pb.N, pb.Kp, bn / 2));
+    T4R_TRY(make_tmap(&bl2, pb.b_planes + pb.b_rows * pb.Kp, pb.N, pb.Kp, bn / 2));
     const int64_t pair_tiles = ((pb.M + 2 * BM - 1) / (2 * BM)) * ((pb.N + bn - 1) / bn);
     // the head kernel that keeps the A tile in shared memory (the head entry point decided it: head_resident_partials)
     T4R_REQUIRE(!ep.head_resident || (ep.head && bn == 256 && dp.nkb <= HeadResCfg::MAX_KB),
@@ -1788,42 +1674,25 @@ int launch_gemm(const GemmProblem& pb, const GemmEpilogue& ep, cudaStream_t stre
       if (bn == 128) return launch_inst2<128, true, false>(ah, al, bh2, bl2, dp, pair_tiles, stream);
       return launch_inst2<64, true, false>(ah, al, bh2, bl2, dp, pair_tiles, stream);
     }
-    // planes-only dense output (the Q|K|V projection): TMA stores instead of per-lane global stores (T4R_GEMM_TMA_STORE)
-    int tma_store = T4R_GEMM_TMA_STORE_DEFAULT;
-    if (const char* e = getenv("T4R_GEMM_TMA_STORE")) tma_store = atoi(e);
-    if (tma_store && bn == 256 && ep.out_planes && !ep.out_f32 && !ep.out_pre && !ep.residual && !ep.residual_planes &&
-        !ep.row_code && !ep.col_scale && pb.m_dev == nullptr && pb.N % 32 == 0 && ep.ldpl % 8 == 0 &&
-        (reinterpret_cast<uintptr_t>(ep.out_planes) & 15) == 0 && (ep.plane_stride * 2) % 16 == 0 && dp.ep.debug == 0) {
-      CUtensorMap oh, ol;
-      T4R_TRY(make_tmap(&oh, ep.out_planes, pb.M, ep.ldpl, 32, 64));
-      T4R_TRY(make_tmap(&ol, ep.out_planes + ep.plane_stride, pb.M, ep.ldpl, 32, 64));
-      return launch_inst2<256, false, false, true>(ah, al, bh2, bl2, dp, pair_tiles, stream, &oh, &ol);
-    }
     if (bn == 256) return launch_inst2<256, false, false>(ah, al, bh2, bl2, dp, pair_tiles, stream);
     if (bn == 128) return launch_inst2<128, false, false>(ah, al, bh2, bl2, dp, pair_tiles, stream);
     return launch_inst2<64, false, false>(ah, al, bh2, bl2, dp, pair_tiles, stream);
   }
 
-  T4R_REQUIRE(!ep.head_resident, "gemm: resident head needs the CTA-pair path (T4R_GEMM_2CTA=1, 128-byte rows, M > 128)");
-#define T4R_GEMM_DISPATCH(RBV)                                                                              \
-  do {                                                                                                      \
-    if (ep.head) {                                                                                          \
-      if (bn == 256) return launch_inst<256, false, true, RBV>(ah, al, bh, bl, dp, max_tiles, stream);      \
-      if (bn == 128) return launch_inst<128, false, true, RBV>(ah, al, bh, bl, dp, max_tiles, stream);      \
-      return launch_inst<64, false, true, RBV>(ah, al, bh, bl, dp, max_tiles, stream);                      \
-    }                                                                                                       \
-    if (ln) {                                                                                               \
-      if (bn == 256) return launch_inst<256, true, false, RBV>(ah, al, bh, bl, dp, max_tiles, stream);      \
-      if (bn == 128) return launch_inst<128, true, false, RBV>(ah, al, bh, bl, dp, max_tiles, stream);      \
-      return launch_inst<64, true, false, RBV>(ah, al, bh, bl, dp, max_tiles, stream);                      \
-    }                                                                                                       \
-    if (bn == 256) return launch_inst<256, false, false, RBV>(ah, al, bh, bl, dp, max_tiles, stream);       \
-    if (bn == 128) return launch_inst<128, false, false, RBV>(ah, al, bh, bl, dp, max_tiles, stream);       \
-    return launch_inst<64, false, false, RBV>(ah, al, bh, bl, dp, max_tiles, stream);                       \
-  } while (0)
-  if (rb == 64) T4R_GEMM_DISPATCH(64);
-  T4R_GEMM_DISPATCH(128);
-#undef T4R_GEMM_DISPATCH
+  T4R_REQUIRE(!ep.head_resident, "gemm: resident head needs the CTA-pair path (T4R_GEMM_2CTA=1, M > 128)");
+  if (ep.head) {
+    if (bn == 256) return launch_inst<256, false, true>(ah, al, bh, bl, dp, max_tiles, stream);
+    if (bn == 128) return launch_inst<128, false, true>(ah, al, bh, bl, dp, max_tiles, stream);
+    return launch_inst<64, false, true>(ah, al, bh, bl, dp, max_tiles, stream);
+  }
+  if (ln) {
+    if (bn == 256) return launch_inst<256, true, false>(ah, al, bh, bl, dp, max_tiles, stream);
+    if (bn == 128) return launch_inst<128, true, false>(ah, al, bh, bl, dp, max_tiles, stream);
+    return launch_inst<64, true, false>(ah, al, bh, bl, dp, max_tiles, stream);
+  }
+  if (bn == 256) return launch_inst<256, false, false>(ah, al, bh, bl, dp, max_tiles, stream);
+  if (bn == 128) return launch_inst<128, false, false>(ah, al, bh, bl, dp, max_tiles, stream);
+  return launch_inst<64, false, false>(ah, al, bh, bl, dp, max_tiles, stream);
 }
 
 
@@ -1858,30 +1727,16 @@ struct FfnDev {
 
 constexpr int FFN_HC = 128;                 // hidden units per chunk
 constexpr int FFN_STAGE_BYTES = 64 * 1024;  // one ring stage (see below)
-#ifndef T4R_FFN_STAGES
-#define T4R_FFN_STAGES 3
-#endif
-constexpr int FFN_STAGES = T4R_FFN_STAGES;
-constexpr int FFN_SMEM_BYTES = FFN_STAGES * FFN_STAGE_BYTES + 1024 + 256 + 4096 + 8 * 32 * 20 * 4;   // CTA-pair variant
+constexpr int FFN_STAGES = 3;
+constexpr int FFN_SMEM_BYTES = FFN_STAGES * FFN_STAGE_BYTES + 1024 + 256 + 4096 + 8 * 32 * 20 * 4;
 
-// NG = column groups of the epilogue (4 NG epilogue warps): 2 = the original eight warps, 4 = sixteen (each warp then
-// GELUs 32 instead of 64 hidden units of a chunk and owns D / 4 instead of D / 2 columns of the final LayerNorm
-// epilogue).  Sixteen warps need 40 KB of staging tiles: the operand ring drops to two 64 KB stages (FfnCfg).
-template <int NG>
-struct FfnCfg {
-  static constexpr int STAGES = (NG == 2) ? FFN_STAGES : 2;
-  static constexpr int THREADS = (2 + 4 * NG) * 32;
-  static constexpr int XCH_BYTES = 2 * NG * 128 * 8;
-  static constexpr int SMEM_BYTES = STAGES * FFN_STAGE_BYTES + 1024 + 256 + XCH_BYTES + 4 * NG * 32 * 20 * 4;
-};
-
-template <int D, int NG>
-__global__ void __launch_bounds__(FfnCfg<NG>::THREADS, 1)
+template <int D>
+__global__ void __launch_bounds__(320, 1)
 ffn_fused_kernel(const __grid_constant__ CUtensorMap tmXh, const __grid_constant__ CUtensorMap tmXl,
                  const __grid_constant__ CUtensorMap tmW1h, const __grid_constant__ CUtensorMap tmW1l,
                  const __grid_constant__ CUtensorMap tmW2h, const __grid_constant__ CUtensorMap tmW2l, const FfnDev p) {
-  constexpr int STAGES = FfnCfg<NG>::STAGES;
-  constexpr int HCW = FFN_HC / NG;                  // hidden units of a chunk per epilogue warp
+  constexpr int STAGES = FFN_STAGES;
+  constexpr int HCW = FFN_HC / 2;                   // hidden units of a chunk per epilogue warp
   constexpr int KB1 = D / 64;                       // k blocks of GEMM1 (K = d)
   constexpr int KB2 = FFN_HC / 64;                  // k blocks of GEMM2 per chunk (K = 128)
   constexpr int XP = BM * 128;                      // X plane bytes per k block
@@ -1900,7 +1755,7 @@ ffn_fused_kernel(const __grid_constant__ CUtensorMap tmXh, const __grid_constant
   uint64_t* y_empty = y_full + 1;
   uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(y_empty + 1);
   float2* xch = reinterpret_cast<float2*>(smem + STAGES * FFN_STAGE_BYTES + 256);
-  float* stg_all = reinterpret_cast<float*>(smem + STAGES * FFN_STAGE_BYTES + 256 + FfnCfg<NG>::XCH_BYTES);
+  float* stg_all = reinterpret_cast<float*>(smem + STAGES * FFN_STAGE_BYTES + 256 + 4096);
 
   const int warp = warp_id();
   const int lane = lane_id();
@@ -1914,9 +1769,9 @@ ffn_fused_kernel(const __grid_constant__ CUtensorMap tmXh, const __grid_constant
   }
   if (warp == 1 && lane == 0) {
     for (int i = 0; i < STAGES; ++i) { mbar_init(&full_bar[i], 1); mbar_init(&empty_bar[i], 1); }
-    mbar_init(s_full, 1); mbar_init(s_empty, 4 * NG);
-    mbar_init(g_full, 4 * NG); mbar_init(g_empty, 1);
-    mbar_init(y_full, 1); mbar_init(y_empty, 4 * NG);
+    mbar_init(s_full, 1); mbar_init(s_empty, 8);
+    mbar_init(g_full, 8); mbar_init(g_empty, 1);
+    mbar_init(y_full, 1); mbar_init(y_empty, 8);
     fence_barrier_init();
   }
   if (warp == 2) {
@@ -2033,9 +1888,9 @@ ffn_fused_kernel(const __grid_constant__ CUtensorMap tmXh, const __grid_constant
     }
     __syncwarp();
   } else {
-    // ===================== epilogue warps (2 .. 1 + 4 NG) =====================
+    // ===================== epilogue warps (2..9) =====================
     const int quad = warp & 3;
-    const int half = (warp - 2) >> 2;   // column group 0 .. NG-1
+    const int half = (warp - 2) >> 2;   // which half of the hidden chunk and of the output columns
     const uint32_t lane_base = static_cast<uint32_t>(quad * 32) << 16;
     uint32_t ph_s_full = 0, ph_g_empty = 0, ph_y_full = 0, tile_parity = 0;
     GemmDev gp;  // view of the final epilogue for epilogue_dense
@@ -2099,9 +1954,9 @@ ffn_fused_kernel(const __grid_constant__ CUtensorMap tmXh, const __grid_constant
       {
         const int64_t left = static_cast<int64_t>(p.M) - row0;
         const int rows_valid = left < 0 ? 0 : (left > 32 ? 32 : static_cast<int>(left));
-        float2* xg0 = xch + (tile_parity * NG) * 128 + quad * 32 + lane;   // [parity][group][row]
-        epilogue_dense<D, true, NG>(gp, tmem_base + lane_base + Y_COL + half * (D / NG), row0, rows_valid, lane,
-                                    static_cast<int64_t>(half) * (D / NG), stg_all + (warp - 2) * STG_WORDS, xg0, half);
+        float2* xg0 = xch + (tile_parity * 2) * 128 + quad * 32 + lane;   // [parity][group][row]
+        epilogue_dense<D, true>(gp, tmem_base + lane_base + Y_COL + half * (D / 2), row0, rows_valid, lane,
+                                static_cast<int64_t>(half) * (D / 2), stg_all + (warp - 2) * STG_WORDS, xg0, half);
         tile_parity ^= 1;
       }
       tc_fence_before_sync();
@@ -2117,312 +1972,38 @@ ffn_fused_kernel(const __grid_constant__ CUtensorMap tmXh, const __grid_constant
   if (warp == 2) tmem_dealloc(tmem_base, 512);
 }
 
-template <int D, int NG>
+template <int D>
 static int launch_ffn_inst(const CUtensorMap (&tm)[6], const FfnDev& dp, cudaStream_t stream) {
-  auto kern = ffn_fused_kernel<D, NG>;
+  auto kern = ffn_fused_kernel<D>;
   static bool attr_set = false;
   if (!attr_set) {
-    T4R_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, FfnCfg<NG>::SMEM_BYTES));
+    T4R_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, FFN_SMEM_BYTES));
     attr_set = true;
   }
   const int tiles = (dp.M + BM - 1) / BM;
   const int grid = tiles < num_sms() ? tiles : num_sms();
-  kern<<<grid, FfnCfg<NG>::THREADS, FfnCfg<NG>::SMEM_BYTES, stream>>>(tm[0], tm[1], tm[2], tm[3], tm[4], tm[5], dp);
+  kern<<<grid, 320, FFN_SMEM_BYTES, stream>>>(tm[0], tm[1], tm[2], tm[3], tm[4], tm[5], dp);
   T4R_LAUNCH_CHECK("ffn_fused_kernel");
   return 0;
 }
 
-
-// ----------------------------------------------------------------------------
-// CTA-pair variant of the fused feed-forward (cta_group::2, 256 rows per pair): each CTA streams its own 128 rows
-// of X but only HALF of every W1 / W2 chunk, so the weight stream per SM halves.  Same schedule as
-// ffn_fused_kernel; the six hand-off barriers live in the leader (rank 0) for the epilogue -> MMA direction
-// (s_empty, g_full, y_empty: 16 arrivals = 8 warps x 2 CTAs) and are multicast to both CTAs for the MMA -> epilogue
-// direction (s_full, g_empty, y_full).  GEMM2 takes its A operand (the GELU'd chunk) from each CTA's own TMEM.
-// ----------------------------------------------------------------------------
-__device__ __forceinline__ void umma_bf16_ts_pair(uint32_t tmem_d, uint32_t tmem_a, uint64_t bdesc, uint32_t idesc,
-                                                  uint32_t accumulate) {
-  asm volatile(
-      "{\n\t.reg .pred p;\n\t"
-      "setp.ne.b32 p, %4, 0;\n\t"
-      "tcgen05.mma.cta_group::2.kind::f16 [%0], [%1], %2, %3, p;\n\t}"
-      ::"r"(tmem_d), "r"(tmem_a), "l"(bdesc), "r"(idesc), "r"(accumulate)
-      : "memory");
-}
-
-constexpr int FFN2_STAGE_BYTES = 48 * 1024;  // GEMM1: X kb hi/lo (2 x 16 KB) + half W1 chunk hi/lo (2 x 8 KB); GEMM2: half W2 hi/lo (2 x 16 KB at d = 256)
-constexpr int FFN2_STAGES = 4;
-constexpr int FFN2_SMEM_BYTES = FFN2_STAGES * FFN2_STAGE_BYTES + 1024 + 256 + 4096 + 8 * 32 * 20 * 4;
-
-template <int D>
-__global__ void __launch_bounds__(320, 1)
-ffn_fused2_kernel(const __grid_constant__ CUtensorMap tmXh, const __grid_constant__ CUtensorMap tmXl,
-                  const __grid_constant__ CUtensorMap tmW1h, const __grid_constant__ CUtensorMap tmW1l,
-                  const __grid_constant__ CUtensorMap tmW2h, const __grid_constant__ CUtensorMap tmW2l, const FfnDev p) {
-  constexpr int KB1 = D / 64;
-  constexpr int KB2 = FFN_HC / 64;
-  constexpr int XP = BM * 128;                // X plane bytes per k block (own 128 rows)
-  constexpr int W1P = (FFN_HC / 2) * 128;     // this CTA's half of the W1 chunk
-  constexpr int W2P = (D / 2) * 128;          // this CTA's half of the W2 chunk
-  constexpr uint32_t Y_COL = 0, S_COL = 256, GH_COL = 384, GL_COL = 448;
-  extern __shared__ uint8_t smem_raw[];
-  uint8_t* smem = smem_raw + ((1024u - (smem_u32(smem_raw) & 1023u)) & 1023u);
-  uint64_t* full_bar = reinterpret_cast<uint64_t*>(smem + FFN2_STAGES * FFN2_STAGE_BYTES);
-  uint64_t* empty_bar = full_bar + FFN2_STAGES;
-  uint64_t* s_full = empty_bar + FFN2_STAGES;
-  uint64_t* s_empty = s_full + 1;
-  uint64_t* g_full = s_empty + 1;
-  uint64_t* g_empty = g_full + 1;
-  uint64_t* y_full = g_empty + 1;
-  uint64_t* y_empty = y_full + 1;
-  uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(y_empty + 1);
-  float2* xch = reinterpret_cast<float2*>(smem + FFN2_STAGES * FFN2_STAGE_BYTES + 256);
-  float* stg_all = reinterpret_cast<float*>(smem + FFN2_STAGES * FFN2_STAGE_BYTES + 256 + 4096);
-
-  const int warp = warp_id();
-  const int lane = lane_id();
-  const int rank = static_cast<int>(cluster_ctarank());
-  const bool leader = (rank == 0);
-  const int pair = blockIdx.x >> 1;
-  const int npairs = gridDim.x >> 1;
-  const int tiles_m = (p.M + 2 * BM - 1) / (2 * BM);
-  const int NC = p.n_chunks;
-
-  if (warp == 0 && lane == 0) {
-    tma_prefetch_desc(&tmXh); tma_prefetch_desc(&tmXl);
-    tma_prefetch_desc(&tmW1h); tma_prefetch_desc(&tmW1l);
-    tma_prefetch_desc(&tmW2h); tma_prefetch_desc(&tmW2l);
-  }
-  if (warp == 1 && lane == 0) {
-    for (int i = 0; i < FFN2_STAGES; ++i) { mbar_init(&full_bar[i], 1); mbar_init(&empty_bar[i], 1); }
-    mbar_init(s_full, 1); mbar_init(s_empty, 16);
-    mbar_init(g_full, 16); mbar_init(g_empty, 1);
-    mbar_init(y_full, 1); mbar_init(y_empty, 16);
-    fence_barrier_init();
-  }
-  if (warp == 2) {
-    tmem_alloc_pair(tmem_slot, 512);
-    tmem_relinquish_pair();
-  }
-  tc_fence_before_sync();
-  __syncthreads();
-  cluster_sync_all();
-  tc_fence_after_sync();
-  const uint32_t tmem_base = *tmem_slot;
-
-  if (warp == 0) {
-    // ===================== TMA producer (both CTAs; bytes credited to the leader's full barrier) =====
-    if (lane == 0) {
-      int stage = 0;
-      uint32_t phase = 0;
-      auto load_g1 = [&](int m0, int c, int kb) {
-        mbar_wait(&empty_bar[stage], phase ^ 1);
-        uint8_t* st = smem + stage * FFN2_STAGE_BYTES;
-        if (leader) mbar_arrive_expect_tx(&full_bar[stage], 2 * (2 * XP + 2 * W1P));
-        tma_load_2d_pair(st, &tmXh, &full_bar[stage], kb * 64, m0);
-        tma_load_2d_pair(st + XP, &tmXl, &full_bar[stage], kb * 64, m0);
-        tma_load_2d_pair(st + 2 * XP, &tmW1h, &full_bar[stage], kb * 64, c * FFN_HC + rank * (FFN_HC / 2));
-        tma_load_2d_pair(st + 2 * XP + W1P, &tmW1l, &full_bar[stage], kb * 64, c * FFN_HC + rank * (FFN_HC / 2));
-        if (++stage == FFN2_STAGES) { stage = 0; phase ^= 1; }
-      };
-      auto load_g2 = [&](int c, int kb) {
-        mbar_wait(&empty_bar[stage], phase ^ 1);
-        uint8_t* st = smem + stage * FFN2_STAGE_BYTES;
-        if (leader) mbar_arrive_expect_tx(&full_bar[stage], 2 * (2 * W2P));
-        tma_load_2d_pair(st, &tmW2h, &full_bar[stage], c * FFN_HC + kb * 64, rank * (D / 2));
-        tma_load_2d_pair(st + W2P, &tmW2l, &full_bar[stage], c * FFN_HC + kb * 64, rank * (D / 2));
-        if (++stage == FFN2_STAGES) { stage = 0; phase ^= 1; }
-      };
-      for (int tile = pair; tile < tiles_m; tile += npairs) {
-        const int m0 = tile * (2 * BM) + rank * BM;
-        for (int kb = 0; kb < KB1; ++kb) load_g1(m0, 0, kb);
-        for (int c = 0; c < NC; ++c) {
-          if (c + 1 < NC)
-            for (int kb = 0; kb < KB1; ++kb) load_g1(m0, c + 1, kb);
-          for (int kb = 0; kb < KB2; ++kb) load_g2(c, kb);
-        }
-      }
-    }
-    __syncwarp();
-  } else if (warp == 1) {
-    // ===================== MMA issuer (leader only) =====================
-    if (leader && lane == 0) {
-      constexpr uint32_t idesc1 = umma_idesc_bf16(2 * BM, FFN_HC);
-      constexpr uint32_t idesc2 = umma_idesc_bf16(2 * BM, D);
-      int stage = 0;
-      uint32_t phase = 0;
-      uint32_t ph_s_empty = 0, ph_g_full = 0, ph_y_empty = 0;
-      auto gemm1 = [&]() {
-        mbar_wait(s_empty, ph_s_empty ^ 1);
-        ph_s_empty ^= 1;
-        tc_fence_after_sync();
-        for (int kb = 0; kb < KB1; ++kb) {
-          mbar_wait(&full_bar[stage], phase);
-          tc_fence_after_sync();
-          const uint32_t a_hi = smem_u32(smem + stage * FFN2_STAGE_BYTES);
-          const uint32_t a_lo = a_hi + XP, b_hi = a_hi + 2 * XP, b_lo = b_hi + W1P;
-          if (!(p.ep.debug & 4))
-#pragma unroll
-          for (int k4 = 0; k4 < 4; ++k4) {
-            umma_bf16_pair(tmem_base + S_COL, umma_desc_sw128(a_lo + k4 * 32), umma_desc_sw128(b_hi + k4 * 32), idesc1, (kb | k4) != 0);
-            umma_bf16_pair(tmem_base + S_COL, umma_desc_sw128(a_hi + k4 * 32), umma_desc_sw128(b_lo + k4 * 32), idesc1, 1u);
-            umma_bf16_pair(tmem_base + S_COL, umma_desc_sw128(a_hi + k4 * 32), umma_desc_sw128(b_hi + k4 * 32), idesc1, 1u);
-          }
-          umma_commit_pair(&empty_bar[stage]);
-          if (++stage == FFN2_STAGES) { stage = 0; phase ^= 1; }
-        }
-        umma_commit_pair(s_full);
-      };
-      for (int tile = pair; tile < tiles_m; tile += npairs) {
-        gemm1();
-        for (int c = 0; c < NC; ++c) {
-          if (c + 1 < NC) gemm1();
-          mbar_wait(g_full, ph_g_full);
-          ph_g_full ^= 1;
-          if (c == 0) {
-            mbar_wait(y_empty, ph_y_empty ^ 1);
-            ph_y_empty ^= 1;
-          }
-          tc_fence_after_sync();
-          for (int kb = 0; kb < KB2; ++kb) {
-            mbar_wait(&full_bar[stage], phase);
-            tc_fence_after_sync();
-            const uint32_t b_hi = smem_u32(smem + stage * FFN2_STAGE_BYTES);
-            const uint32_t b_lo = b_hi + W2P;
-            if (!(p.ep.debug & 8))
-#pragma unroll
-            for (int k4 = 0; k4 < 4; ++k4) {
-              const uint32_t acol = static_cast<uint32_t>(kb * 32 + k4 * 8);
-              umma_bf16_ts_pair(tmem_base + Y_COL, tmem_base + GL_COL + acol, umma_desc_sw128(b_hi + k4 * 32), idesc2, (c | kb | k4) != 0);
-              umma_bf16_ts_pair(tmem_base + Y_COL, tmem_base + GH_COL + acol, umma_desc_sw128(b_lo + k4 * 32), idesc2, 1u);
-              umma_bf16_ts_pair(tmem_base + Y_COL, tmem_base + GH_COL + acol, umma_desc_sw128(b_hi + k4 * 32), idesc2, 1u);
-            }
-            umma_commit_pair(&empty_bar[stage]);
-            if (++stage == FFN2_STAGES) { stage = 0; phase ^= 1; }
-          }
-          umma_commit_pair(g_empty);
-          if (c == NC - 1) umma_commit_pair(y_full);
-        }
-      }
-    }
-    __syncwarp();
-  } else {
-    // ===================== epilogue warps (2..9) of both CTAs =====================
-    const int quad = warp & 3;
-    const int half = (warp - 2) >> 2;
-    const uint32_t lane_base = static_cast<uint32_t>(quad * 32) << 16;
-    uint32_t ph_s_full = 0, ph_g_empty = 0, ph_y_full = 0, tile_parity = 0;
-    GemmDev gp;
-    gp.M = p.M; gp.N = D; gp.nkb = 0; gp.nprod = 3; gp.m_dev = nullptr; gp.ep = p.ep;
-    for (int tile = pair; tile < tiles_m; tile += npairs) {
-      const int64_t row0 = static_cast<int64_t>(tile) * (2 * BM) + rank * BM + quad * 32;
-      for (int c = 0; c < NC; ++c) {
-        mbar_wait(s_full, ph_s_full);
-        ph_s_full ^= 1;
-        tc_fence_after_sync();
-        float v[64];
-        tmem_ld<64>(tmem_base + lane_base + S_COL + half * 64, v);
-        tc_fence_before_sync();
-        __syncwarp();
-        if (lane == 0) mbar_arrive_leader(s_empty);
-        const float* b1 = p.b1 + c * FFN_HC + half * 64;
-        uint32_t gh[32], gl[32];
-#pragma unroll
-        for (int j = 0; j < 16; ++j) {  // bias + GELU + hi/lo split on packed fp32 pairs (fma.rn.f32x2)
-          const float4 b = __ldg(reinterpret_cast<const float4*>(b1) + j);
-          const float2 g0 = gelu_erf2(__fadd2_rn(make_float2(v[4 * j + 0], v[4 * j + 1]), make_float2(b.x, b.y)));
-          const float2 g1 = gelu_erf2(__fadd2_rn(make_float2(v[4 * j + 2], v[4 * j + 3]), make_float2(b.z, b.w)));
-          split_bf16x2(g0, gh[2 * j], gl[2 * j]);
-          split_bf16x2(g1, gh[2 * j + 1], gl[2 * j + 1]);
-        }
-        mbar_wait(g_empty, ph_g_empty ^ 1);
-        ph_g_empty ^= 1;
-        tc_fence_after_sync();
-#pragma unroll
-        for (int q = 0; q < 4; ++q) {
-          uint32_t r[8];
-#pragma unroll
-          for (int j = 0; j < 8; ++j) r[j] = gh[q * 8 + j];
-          tmem_st8(tmem_base + lane_base + GH_COL + half * 32 + q * 8, r);
-#pragma unroll
-          for (int j = 0; j < 8; ++j) r[j] = gl[q * 8 + j];
-          tmem_st8(tmem_base + lane_base + GL_COL + half * 32 + q * 8, r);
-        }
-        tmem_st_wait();
-        tc_fence_before_sync();
-        __syncwarp();
-        if (lane == 0) mbar_arrive_leader(g_full);
-      }
-      mbar_wait(y_full, ph_y_full);
-      ph_y_full ^= 1;
-      tc_fence_after_sync();
-      {
-        const int64_t left = static_cast<int64_t>(p.M) - row0;
-        const int rows_valid = left < 0 ? 0 : (left > 32 ? 32 : static_cast<int>(left));
-        float2* xg0 = xch + (tile_parity * 2) * 128 + quad * 32 + lane;   // [parity][group][row]
-        epilogue_dense<D, true>(gp, tmem_base + lane_base + Y_COL + half * (D / 2), row0, rows_valid, lane,
-                                static_cast<int64_t>(half) * (D / 2), stg_all + (warp - 2) * STG_WORDS, xg0, half);
-        tile_parity ^= 1;
-      }
-      tc_fence_before_sync();
-      __syncwarp();
-      if (lane == 0) mbar_arrive_leader(y_empty);
-    }
-  }
-
-  tc_fence_before_sync();
-  __syncthreads();
-  cluster_sync_all();
-  tc_fence_after_sync();
-  if (warp == 2) tmem_dealloc_pair(tmem_base, 512);
-}
-
-template <int D>
-static int launch_ffn2_inst(const CUtensorMap (&tm)[6], const FfnDev& dp, cudaStream_t stream) {
-  auto kern = ffn_fused2_kernel<D>;
-  static bool attr_set = false;
-  if (!attr_set) {
-    T4R_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, FFN2_SMEM_BYTES));
-    attr_set = true;
-  }
-  const int pair_tiles = (dp.M + 2 * BM - 1) / (2 * BM);
-  const int max_pairs = num_sms() / 2;
-  const int pairs = pair_tiles < max_pairs ? pair_tiles : max_pairs;
-  cudaLaunchConfig_t cfg = {};
-  cfg.gridDim = dim3(2 * pairs, 1, 1);
-  cfg.blockDim = dim3(320, 1, 1);
-  cfg.dynamicSmemBytes = FFN2_SMEM_BYTES;
-  cfg.stream = stream;
-  cudaLaunchAttribute attr[1];
-  attr[0].id = cudaLaunchAttributeClusterDimension;
-  attr[0].val.clusterDim.x = 2;
-  attr[0].val.clusterDim.y = 1;
-  attr[0].val.clusterDim.z = 1;
-  cfg.attrs = attr;
-  cfg.numAttrs = 1;
-  T4R_CUDA(cudaLaunchKernelEx(&cfg, kern, tm[0], tm[1], tm[2], tm[3], tm[4], tm[5], dp));
-  T4R_LAUNCH_CHECK("ffn_fused2_kernel");
-  return 0;
-}
 
 bool ffn_fused_supported(int d, int hidden) { return (d == 64 || d == 128 || d == 256) && hidden % FFN_HC == 0; }
 
 // x_planes [2, M, d], w1_planes [2, hidden, d], w2_planes [2, d, hidden]; `ep` = final epilogue (bias = b2,
 // residual / residual_planes, ln_gamma/beta/eps, out_f32 / out_pre / out_planes, all with row length d).
 int launch_ffn_fused(const __nv_bfloat16* x_planes, int64_t M, int d, int hidden, const __nv_bfloat16* w1_planes,
-                     const float* b1, const __nv_bfloat16* w2_planes, const GemmEpilogue& ep, cudaStream_t stream,
-                     int64_t x_plane_stride) {
+                     const float* b1, const __nv_bfloat16* w2_planes, const GemmEpilogue& ep, cudaStream_t stream) {
   T4R_REQUIRE(ffn_fused_supported(d, hidden), "ffn_fused: unsupported d=%d hidden=%d", d, hidden);
   T4R_REQUIRE(ep.ln_gamma && ep.ln_beta && b1, "ffn_fused: needs b1 and a LayerNorm epilogue");
   T4R_REQUIRE(M > 0 && M < (1ll << 31), "ffn_fused: bad M");
-  if (x_plane_stride <= 0) x_plane_stride = M * d;   // elements between the hi and the lo plane of X
   CUtensorMap tm[6];
-  T4R_TRY(make_tmap(&tm[0], x_planes, M, d, BM, 128));
-  T4R_TRY(make_tmap(&tm[1], x_planes + x_plane_stride, M, d, BM, 128));
-  T4R_TRY(make_tmap(&tm[2], w1_planes, hidden, d, FFN_HC, 128));
-  T4R_TRY(make_tmap(&tm[3], w1_planes + static_cast<int64_t>(hidden) * d, hidden, d, FFN_HC, 128));
-  T4R_TRY(make_tmap(&tm[4], w2_planes, d, hidden, d, 128));
-  T4R_TRY(make_tmap(&tm[5], w2_planes + static_cast<int64_t>(d) * hidden, d, hidden, d, 128));
+  T4R_TRY(make_tmap(&tm[0], x_planes, M, d, BM));
+  T4R_TRY(make_tmap(&tm[1], x_planes + M * d, M, d, BM));
+  T4R_TRY(make_tmap(&tm[2], w1_planes, hidden, d, FFN_HC));
+  T4R_TRY(make_tmap(&tm[3], w1_planes + static_cast<int64_t>(hidden) * d, hidden, d, FFN_HC));
+  T4R_TRY(make_tmap(&tm[4], w2_planes, d, hidden, d));
+  T4R_TRY(make_tmap(&tm[5], w2_planes + static_cast<int64_t>(d) * hidden, d, hidden, d));
   FfnDev dp;
   dp.M = static_cast<int>(M);
   dp.n_chunks = hidden / FFN_HC;
@@ -2433,27 +2014,9 @@ int launch_ffn_fused(const __nv_bfloat16* x_planes, int64_t M, int d, int hidden
     if (dbg < 0) { const char* e = getenv("T4R_GEMM_DEBUG"); dbg = e ? atoi(e) : 0; }
     dp.ep.debug = dbg & (1 | 2 | 4 | 8 | 64);
   }
-  int two_cta = T4R_FFN_2CTA_DEFAULT;  // measured slower than the single-CTA kernel (DESIGN.md): opt-in, kept parity-tested
-  if (const char* e = getenv("T4R_FFN_2CTA")) two_cta = atoi(e);
-  if (two_cta && M > BM) {  // CTA pairs: each CTA streams half of every weight chunk
-    CUtensorMap t2[6] = {tm[0], tm[1], tm[2], tm[3], tm[4], tm[5]};
-    T4R_TRY(make_tmap(&t2[2], w1_planes, hidden, d, FFN_HC / 2, 128));
-    T4R_TRY(make_tmap(&t2[3], w1_planes + static_cast<int64_t>(hidden) * d, hidden, d, FFN_HC / 2, 128));
-    T4R_TRY(make_tmap(&t2[4], w2_planes, d, hidden, d / 2, 128));
-    T4R_TRY(make_tmap(&t2[5], w2_planes + static_cast<int64_t>(d) * hidden, d, hidden, d / 2, 128));
-    if (d == 256) return launch_ffn2_inst<256>(t2, dp, stream);
-    if (d == 128) return launch_ffn2_inst<128>(t2, dp, stream);
-    return launch_ffn2_inst<64>(t2, dp, stream);
-  }
-  // T4R_FFN_EPW: epilogue warps of the fused kernel, 8 or 16 (16: each warp's share of the GELU chunk and of the
-  // final LayerNorm epilogue halves; d >= 128 only: a LayerNorm chunk is 32 columns wide)
-  int epw = T4R_FFN_EPW_DEFAULT;
-  if (const char* e = getenv("T4R_FFN_EPW")) epw = atoi(e);
-  if (epw == 16 && d == 256) return launch_ffn_inst<256, 4>(tm, dp, stream);
-  if (epw == 16 && d == 128) return launch_ffn_inst<128, 4>(tm, dp, stream);
-  if (d == 256) return launch_ffn_inst<256, 2>(tm, dp, stream);
-  if (d == 128) return launch_ffn_inst<128, 2>(tm, dp, stream);
-  return launch_ffn_inst<64, 2>(tm, dp, stream);
+  if (d == 256) return launch_ffn_inst<256>(tm, dp, stream);
+  if (d == 128) return launch_ffn_inst<128>(tm, dp, stream);
+  return launch_ffn_inst<64>(tm, dp, stream);
 }
 
 }  // namespace t4r

@@ -107,8 +107,7 @@ int head_resident_partials(int64_t M, int64_t V, int Kp);  // > 0: the resident-
 // fused feed-forward block (t4r_gemm.cu): Y = epilogue(gelu(X W1^T + b1) W2^T), intermediate kept in TMEM
 bool ffn_fused_supported(int d, int hidden);
 int launch_ffn_fused(const __nv_bfloat16* x_planes, int64_t M, int d, int hidden, const __nv_bfloat16* w1_planes,
-                     const float* b1, const __nv_bfloat16* w2_planes, const GemmEpilogue& ep, cudaStream_t stream,
-                     int64_t x_plane_stride = 0 /* elements between X's hi and lo plane; 0 = M * d */);
+                     const float* b1, const __nv_bfloat16* w2_planes, const GemmEpilogue& ep, cudaStream_t stream);
 
 // ---------------------------------------------------------------------------
 // SIMT kernels (t4r_kernels.cu)

@@ -95,7 +95,7 @@ tsmma_test_kernel(const __grid_constant__ CUtensorMap tmB, const float* __restri
   if (warp == 0) tmem_dealloc(tmem, 512);
 }
 
-int make_tmap_public(CUtensorMap* map, const __nv_bfloat16* base, int64_t rows, int Kp, int box_rows, int rb);
+int make_tmap_public(CUtensorMap* map, const __nv_bfloat16* base, int64_t rows, int Kp, int box_rows);
 
 }  // namespace t4r
 
@@ -104,7 +104,7 @@ extern "C" int t4r_debug_ts_mma(const float* A, const void* b_planes, int N, flo
   using namespace t4r;
   T4R_REQUIRE(A && b_planes && D && (N == 64 || N == 128 || N == 256), "debug_ts_mma: bad arguments");
   CUtensorMap tb;
-  T4R_TRY(make_tmap_public(&tb, static_cast<const __nv_bfloat16*>(b_planes), N, 64, N, 128));
+  T4R_TRY(make_tmap_public(&tb, static_cast<const __nv_bfloat16*>(b_planes), N, 64, N));
   const int smem = N * 128 + 1024 + 64;
   cudaStream_t s = static_cast<cudaStream_t>(stream);
   if (N == 64) {
